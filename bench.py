@@ -1,6 +1,7 @@
 """bench.py -- headline benchmark of the B200-native instance-embedding hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload train|infer|cityscapes|sweep]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -16,7 +17,10 @@ Workloads (BASELINE.json `configs`):
 The default run (N = 1) prints ONE JSON line for `train` that also carries the other three as the extra objects
 "inference", "cityscapes" and "sweep", each with its own value / e2e / roofline / cpu_baseline.
 `value` = whole-job images/s with inputs resident in HBM, `e2e` = the same through the public API with pinned HOST
-buffers (H2D + D2H inside the timed region).
+buffers (H2D + D2H inside the timed region).  `--steps K` is the number of timed steps of every GPU leg.
+`--dump-outputs DIR` writes what the timed path of the workload computed in its last step (train: the metrics, the
+updated parameters and the gradient; infer / cityscapes: softmax, embedding, masks, k-means centres and inertias); the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 `--impl reference` times the reference's CPU implementation of the same workload (oracle/model_ref.py: nn.GRU ReNet,
 the reference's MultiHeadAttention math, its broadcast discriminative-loss graph, real scikit-learn KMeans, cv2) on
 the box's host cores: the FULL batch-16 step as 8 micro-batches of 2 with gradient accumulation, every step it reports timed.
@@ -199,6 +203,31 @@ def _timed_plain(torch):
     return timed
 
 
+DUMP_BUDGET_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: writes each of `arrays` (name -> tensor) as out_dir/<name>.npy, float64 kept, every other dtype as
+    float32, at most DUMP_BUDGET_BYTES in all.  Smaller arrays are written whole; an array above its share of what is left
+    becomes a fixed sample of its flattened elements (seed 0, indices ascending), so runs with the same arguments write
+    files of the same shape that can be compared element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)
+        host[name] = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+    left = DUMP_BUDGET_BYTES - 1024 * len(host)          # room for the .npy headers
+    names = sorted(host, key=lambda n: host[n].nbytes)
+    for i, name in enumerate(names):
+        a = host[name]
+        cap = left // (len(names) - i) // a.itemsize
+        if a.size > cap:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes
+
+
 # ---------------------------------------------------------------------------------------------- clustering parity
 def clustering_parity(pred, model, tens, k, raw_hw, max_images=4, budget_s=100.0, oracle_images=2):
     """Parity of the device clustering on the benchmark images, outside the timed region: bit-exact against the oracle
@@ -282,10 +311,11 @@ def structured_parity(dev, n_cases=3):
 
 
 # ---------------------------------------------------------------------------------------------- inference legs
-def inference_leg(model, dev, peaks, steps, warmup, rank=0, world=1, sampler=None, timed=None, with_cpu=True, shape="cvppp"):
+def inference_leg(model, dev, peaks, steps, warmup, rank=0, world=1, sampler=None, timed=None, with_cpu=True, shape="cvppp",
+                  dump_dir=None):
     """pred.py inference: value (inputs in HBM), e2e (host image in, host masks out), per-kernel times, parity flags
     against the oracle / scikit-learn, and (N = 1) the host-CPU reference beside it.  shape: cvppp (configs[0]) or
-    cityscapes (configs[3])."""
+    cityscapes (configs[3]).  dump_dir: rank 0 writes the last timed step's outputs there (dump_outputs)."""
     import torch
     from isa_b200 import _lib, synth
     from isa_b200.prediction import Prediction
@@ -303,6 +333,7 @@ def inference_leg(model, dev, peaks, steps, warmup, rank=0, world=1, sampler=Non
 
     def step_dev(i):
         sem, emb = model.predict_device(tens[i % n_img])
+        last["net"] = (sem, emb)
         last["o"] = pred.cluster_device(sem[0], emb[0], k, raw_h, raw_w)
 
     def _raw_cycle():
@@ -328,8 +359,11 @@ def inference_leg(model, dev, peaks, steps, warmup, rank=0, world=1, sampler=Non
     clocks = sampler.stop() if sampler is not None else None
     summ = _lib.TIMER.summary()
     launches = sum(_lib.KERNELS_PER_CALL[k_] * c for k_, (c, _) in summ.items())
-    ms_e2e = timed(step_e2e, steps, 1)
     res = last["o"][4]
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {"sem": last["net"][0], "emb": last["net"][1], "fg_mask": last["o"][3],
+                                "ins_mask": last["o"][2], "centers": res.centers, "inertia": res.inertia})
+    ms_e2e = timed(step_e2e, steps, 1)
     n_pts = int(res.info[2])
     it_sum = int(res.n_iter.sum())
     km = summ.get("isa_kmeans_fit", (1, 0.0))
@@ -545,12 +579,12 @@ def run_ours(args):
         if args.no_inference:
             return
         m = fresh_model()
-        out["inference"] = inference_leg(m, dev, peaks, steps=max(args.steps, 20), warmup=max(args.warmup, 3))
+        out["inference"] = inference_leg(m, dev, peaks, steps=args.steps, warmup=args.warmup)
         del m
         torch.cuda.empty_cache()
         try:
             m = fresh_model('Cityscapes')
-            out["cityscapes"] = inference_leg(m, dev, peaks, steps=3, warmup=1, shape="cityscapes")
+            out["cityscapes"] = inference_leg(m, dev, peaks, steps=args.steps, warmup=1, shape="cityscapes")
             del m
         except Exception as e:          # the leg must not take the headline down with it
             out["cityscapes"] = {"error": repr(e)}
@@ -620,6 +654,12 @@ def run_ours(args):
         sampler.start()
         ms = timed(step_dev, args.steps, 3)          # the first warm-up step here captures the graph
         clocks = sampler.stop()
+        if args.dump_outputs and rank == 0:
+            # the step's metrics (the graph's static scalars, overwritten by the next replay) and the parameters and
+            # gradient it left in the optimizer's flat buffers
+            dump = {name.lower().replace(" ", "_"): v for name, v in last["m"].items()}
+            dump.update(params=model.optimizer.flat_param, grad=model.optimizer.flat_grad)
+            dump_outputs(args.dump_outputs, dump)
         ms_e2e = timed(step_e2e, args.steps, 1)
         h2d = sum(t.numel() * t.element_size() for t in host[0])
         # (c) the same step fed the reference collate's int64 one-hot tensors (distilled to label maps on the device)
@@ -664,9 +704,9 @@ def run_ours(args):
             # strict fp32 for the backbone as well (cuDNN TF32 off): what the step costs when NOTHING runs below fp32 accuracy
             torch.backends.cudnn.allow_tf32 = False
             model._graphs.clear(); model._graph_seen.clear()
-            ms_strict = timed(step_dev, max(3, args.steps // 2), 3)
+            ms_strict = timed(step_dev, args.steps, 3)
             torch.backends.cudnn.allow_tf32 = True
-            out["config"]["ms_per_step_cudnn_tf32_off"] = ms_strict / max(3, args.steps // 2)
+            out["config"]["ms_per_step_cudnn_tf32_off"] = ms_strict / args.steps
             del model, devb
             torch.cuda.empty_cache()
             extra_legs(out)
@@ -674,7 +714,7 @@ def run_ours(args):
         city = args.workload == "cityscapes"
         model = fresh_model('Cityscapes' if city else 'CVPPP')
         leg = inference_leg(model, dev, peaks, steps=args.steps, warmup=args.warmup, rank=rank, world=world, sampler=sampler,
-                            timed=timed, with_cpu=False, shape="cityscapes" if city else "cvppp")
+                            timed=timed, with_cpu=False, shape="cityscapes" if city else "cvppp", dump_dir=args.dump_outputs)
         out = {
             "metric": METRIC,
             "value": leg["value"], "unit": "images/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
@@ -854,7 +894,12 @@ def main():
     ap.add_argument("--no-graph", dest="no_graph", action="store_true", help="keep the training step eager (no CUDA-graph replay)")
     ap.add_argument("--no-inference", dest="no_inference", action="store_true",
                     help="train workload: skip the extra legs (inference, cityscapes, sweep, strict fp32) reported at N = 1")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path computed in its last step as DIR/<name>.npy "
+                         "(float32 / float64, at most 64 MB; larger outputs as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "sweep"):
+        ap.error("--dump-outputs needs --impl ours and the train, infer or cityscapes workload")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     _quarantine_stdout()
     if args.impl == "reference":
