@@ -116,8 +116,7 @@ int isa_label_fg_count(const unsigned char* labels, long long total, int K, unsi
  * k-means++ follows scikit-learn's float32 code path decision for decision (float64-upcast candidate distances,
  * candidates by searchsorted on the SEQUENTIAL float32 cumulative sum, float32 potentials).  E-step: packed FP32
  * (fma.rn.f32x2) or, from 33 centres on (C <= 32, k <= 128), tcgen05 MMAs as a filter with an exact pass for the pairs
- * inside the error bound -- both bit-exact with the oracle.  Environment switches (experiments): ISA_KM_TC / ISA_KM_FFMA
- * force the E-step variant, ISA_KM_PRIV, ISA_KM_FLOW, ISA_KM_PPT, ISA_KM_STREAMING select measured alternatives.
+ * inside the error bound -- both bit-exact with the oracle.
  */
 size_t isa_kmeans_workspace_bytes(int ld, int C, int k, int n_init);
 

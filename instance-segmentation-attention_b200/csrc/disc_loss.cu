@@ -1194,7 +1194,7 @@ int isa_disc_loss_fwd(const float* emb, const void* target, int target_kind, con
 
   // ---- label-map forward (one grid barrier, deterministic): label maps, and dense masks that turn out one-hot
   LabParams lp;
-  bool use_lab = !getenv("ISA_DISC_OLD_FWD");
+  bool use_lab = true;
   size_t lab_smem = 0;
   int lab_grid = 0;
   if (use_lab) {

@@ -27,7 +27,6 @@
 #include "isa_ptx.cuh"
 #include "isa_tcgen05.cuh"
 #include <math.h>
-#include <stdlib.h>
 
 namespace {
 
@@ -268,474 +267,6 @@ __global__ void __launch_bounds__(256, 1) gru_scan_bwd_kernel(const GruBwdParams
   }
 }
 
-// ============================================================================================
-// Register-resident variant (the one that runs for the reference's ReNet(.., 100) layers).
-//
-// The generic kernels above keep W_hh in shared memory and stream it through the LSU on every
-// step (one LDS per 3..8 FMAs, 200 active threads): ncu showed them issue- and LDS-latency
-// bound (r1a: 540 us / 882 us per sweep).  Here the recurrent weights live in REGISTERS for the
-// whole sweep and the inner products run on the packed FP32 pipe (fma.rn.f32x2 -> FFMA2: a
-// scalar 3-register FFMA issues every other cycle per scheduler on sm_100, FFMA2 does two FMAs
-// in that slot).  The pairing is along the reduction index: a thread keeps {even-i, odd-i}
-// partial sums, its weights as {w[2k], w[2k+1]} register pairs, and the hidden state sits in
-// shared memory as [i/2][sequence][i%2] so one LDS.128 delivers the operand pairs of two
-// sequences (warp broadcast, no bank conflicts).
-//   forward : thread (unit j, slice ig of IG=5) holds W_hh[g*n+j][20 ig .. 20 ig+20) for the three
-//             gates (60 registers); the IG partial sums meet in shared memory at the thread
-//             that owns (unit j, sequence s), which also keeps h[j][s] in a register;
-//   backward: thread (units p and p+n/2, slice gg of 8) holds 2 x 38 rows of W_hh.
-// The per-step input rows (gx; in backward the gate stash, h_{t-1} and dL/dh rows) are
-// contiguous in the token-major layout, so one warp fetches them two steps ahead with the TMA
-// bulk-copy engine (cp.async.bulk + mbarrier complete_tx): no thread spends registers on
-// prefetching.  S (sequences per CTA) is chosen so that the 2 * n_seq sequence-directions fill
-// the SMs in one wave (S = 14 -> 148 CTAs for the 1024 rows of a batch-16 64x64 map).
-// ============================================================================================
-typedef unsigned long long u64;
-__device__ __forceinline__ void ffma2(u64& acc, u64 a, u64 b) { asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc) : "l"(a), "l"(b)); }
-__device__ __forceinline__ u64 pack2(float lo, float hi) {
-  u64 r;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-  return r;
-}
-__device__ __forceinline__ float sum2(u64 v) {
-  float lo, hi;
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
-  return lo + hi;
-}
-// row stride (floats) of the pair-interleaved [i/2][sequence][2] tiles: 16 B aligned, and RS/4 odd so that the
-// owners' scalar writes (consecutive units = consecutive rows) spread over 8 bank groups
-__host__ __device__ constexpr int pair_row_stride(int S) { return (2 * S) % 8 == 4 ? 2 * S : 2 * S + 4; }
-
-// one pass of the forward partial product over CN sequences starting at C0 (CN in {2,4,6})
-template <int NU, int S, int IRP, int C0, int CN>
-__device__ __forceinline__ void fwd_partial_pass(const u64 (&w)[3][IRP], const float* __restrict__ hp, float* __restrict__ pp) {
-  constexpr int RS = pair_row_stride(S);
-  u64 acc[3][CN];
-#pragma unroll
-  for (int g = 0; g < 3; ++g)
-#pragma unroll
-    for (int s = 0; s < CN; ++s) acc[g][s] = 0ull;
-#pragma unroll
-  for (int k = 0; k < IRP; ++k) {
-    u64 hv[CN];
-#pragma unroll
-    for (int c = 0; c < CN; c += 2) {
-      const ulonglong2 v = *reinterpret_cast<const ulonglong2*>(hp + k * RS + 2 * (C0 + c));
-      hv[c] = v.x; hv[c + 1] = v.y;
-    }
-#pragma unroll
-    for (int s = 0; s < CN; ++s) {
-      ffma2(acc[0][s], w[0][k], hv[s]);
-      ffma2(acc[1][s], w[1][k], hv[s]);
-      ffma2(acc[2][s], w[2][k], hv[s]);
-    }
-  }
-#pragma unroll
-  for (int g = 0; g < 3; ++g)
-#pragma unroll
-    for (int s = 0; s < CN; ++s) pp[((size_t)g * S + C0 + s) * NU] = sum2(acc[g][s]);
-}
-
-template <int NU, int S>
-struct RegFwdCfg {
-  static constexpr int IG = 5;
-  static constexpr int IR = NU / IG;          // reduction slice per thread
-  static constexpr int IRP = IR / 2;          // ... in pairs
-  static constexpr int NT = NU * IG;
-  static constexpr int MI = (S + IG - 1) / IG;
-  static constexpr int STAGES = 2;
-  static constexpr int RS = pair_row_stride(S);
-  static constexpr size_t gx_floats = (size_t)STAGES * S * 3 * NU;
-  static constexpr size_t h_floats = 2 * (size_t)(NU / 2) * RS;
-  static constexpr size_t part_floats = (size_t)IG * 3 * S * NU;
-  static constexpr size_t smem_bytes = (h_floats + part_floats + gx_floats) * sizeof(float) + 16 + 16 * 8;
-};
-
-template <int NU, int S>
-__global__ void __launch_bounds__(RegFwdCfg<NU, S>::NT, 1) gru_fwd_reg_kernel(const GruFwdParams prm) {
-  using Cfg = RegFwdCfg<NU, S>;
-  constexpr int IG = Cfg::IG, IR = Cfg::IR, IRP = Cfg::IRP, MI = Cfg::MI, N3 = 3 * NU, RS = Cfg::RS;
-  static_assert(NU % (2 * IG) == 0 && S <= 16 && S % 2 == 0, "unsupported shape");
-  extern __shared__ __align__(128) float smem[];
-  float* s_gx = smem;                              // [STAGES][S][3n]  (TMA destination, 16 B aligned rows)
-  float* s_h = s_gx + Cfg::gx_floats;              // [2][n/2][RS]: element (i, s) at (i/2)*RS + 2 s + (i & 1)
-  float* s_part = s_h + Cfg::h_floats;             // [IG][3][S][n]
-  uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_part + Cfg::part_floats);
-  long long* s_tok = reinterpret_cast<long long*>(s_bar + 2);   // [S] first token of each sequence (-1: none)
-  const int d = blockIdx.y;
-  const int q0 = blockIdx.x * S;
-  const int T = prm.T;
-  const int tid = threadIdx.x;
-  const int j = tid % NU, ig = tid / NU;
-  const int n_valid = min(S, prm.n_seq - q0);
-
-  if (tid == 0) {
-    mbar_init(&s_bar[0], 1);
-    mbar_init(&s_bar[1], 1);
-    fence_barrier_init();
-  }
-  for (int idx = tid; idx < (int)(Cfg::h_floats + Cfg::gx_floats); idx += Cfg::NT) smem[idx] = 0.f;
-
-  // recurrent weights -> registers (once), as {w[2k], w[2k+1]} pairs
-  u64 w[3][IRP];
-  {
-    const float* __restrict__ wsrc = prm.w_hh + (size_t)d * N3 * NU;
-#pragma unroll
-    for (int g = 0; g < 3; ++g)
-#pragma unroll
-      for (int k = 0; k < IRP; ++k) {
-        const float2 v = __ldg(reinterpret_cast<const float2*>(wsrc + (size_t)(g * NU + j) * NU + ig * IR + 2 * k));
-        w[g][k] = pack2(v.x, v.y);
-      }
-  }
-  const float bhr = __ldg(prm.b_hh + d * N3 + j) + (prm.b_ih ? __ldg(prm.b_ih + d * N3 + j) : 0.f);
-  const float bhz = __ldg(prm.b_hh + d * N3 + NU + j) + (prm.b_ih ? __ldg(prm.b_ih + d * N3 + NU + j) : 0.f);
-  const float bhn = __ldg(prm.b_hh + d * N3 + 2 * NU + j);
-  const float bin = prm.b_ih ? __ldg(prm.b_ih + d * N3 + 2 * NU + j) : 0.f;
-
-  float hreg[MI];
-#pragma unroll
-  for (int m = 0; m < MI; ++m) hreg[m] = 0.f;
-  if (tid < S) s_tok[tid] = tid < n_valid ? tok_base(prm.map, q0 + tid) : -1;
-  __syncthreads();  // barrier init + zero fill visible; generic-proxy writes ordered before the async copies below
-  fence_proxy_async();
-
-  // producer (warp 0): lane s fetches the gx row of sequence s for step `st` into stage st & 1
-  auto issue = [&](int st) {
-    if (tid < 32) {
-      uint64_t* bar = &s_bar[st & 1];
-      if (tid == 0) mbar_arrive_expect_tx(bar, (uint32_t)n_valid * N3 * 4u);
-      __syncwarp();
-      if (tid < n_valid) {
-        const int t = (d == 0) ? st : T - 1 - st;
-        const long long tok = s_tok[tid] + (long long)t * prm.map.t_stride;
-        tma_bulk_g2s(s_gx + ((size_t)(st & 1) * S + tid) * N3, prm.gx + ((size_t)tok * 2 + d) * N3, N3 * 4u, bar);
-      }
-    }
-  };
-  issue(0);
-  if (T > 1) issue(1);
-
-  if constexpr (S >= 8) {
-    // Two sequence groups, A = [0, SA) and B = [SA, S), run half a step apart: while the FP32 pipe works on one
-    // group's matmul the other group's owners do the latency-bound part (partials from shared memory, MUFU gate
-    // math, stores).  Measured 316 -> 288 us per sweep at S = 14; the matmul itself (420 k FMA per step and SM at the
-    // measured 126 FMA/clk/SM) is 3.4 k of the remaining 8.6 k cycles per step.
-    constexpr int SA = (S >= 14) ? 8 : S / 2;
-    float* __restrict__ hbuf = s_h;                       // single buffer: the groups touch disjoint columns
-    const float* __restrict__ hp = hbuf + (size_t)(ig * IRP) * RS;
-    float* __restrict__ pp = s_part + (size_t)(ig * 3) * S * NU + j;
-
-    auto matmul_A = [&]() {
-      if constexpr (SA == 8) { fwd_partial_pass<NU, S, IRP, 0, 4>(w, hp, pp); fwd_partial_pass<NU, S, IRP, 4, 4>(w, hp, pp); }
-      else fwd_partial_pass<NU, S, IRP, 0, SA>(w, hp, pp);
-    };
-    auto matmul_B = [&]() {
-      constexpr int SB = S - SA;
-      if constexpr (SB == 8) { fwd_partial_pass<NU, S, IRP, SA, 4>(w, hp, pp); fwd_partial_pass<NU, S, IRP, SA + 4, 4>(w, hp, pp); }
-      else fwd_partial_pass<NU, S, IRP, SA, SB>(w, hp, pp);
-    };
-    // owners of (unit j, sequence s in [s_lo, s_hi)) at forward step `st`: combine partials, gate math, publish h
-    auto finalize = [&](int st, int s_lo, int s_hi) {
-      const int t = (d == 0) ? st : T - 1 - st;
-      mbar_wait(&s_bar[st & 1], (st >> 1) & 1);
-      const float* __restrict__ gxs = s_gx + (size_t)(st & 1) * S * N3;
-#pragma unroll
-      for (int m = 0; m < MI; ++m) {
-        const int s = ig + IG * m;
-        if (s >= s_lo && s < s_hi) {
-          float ar = bhr, az = bhz, an = bhn;
-#pragma unroll
-          for (int p = 0; p < IG; ++p) {
-            ar += s_part[((size_t)(p * 3 + 0) * S + s) * NU + j];
-            az += s_part[((size_t)(p * 3 + 1) * S + s) * NU + j];
-            an += s_part[((size_t)(p * 3 + 2) * S + s) * NU + j];
-          }
-          const float xr = gxs[s * N3 + j], xz = gxs[s * N3 + NU + j], xn = gxs[s * N3 + 2 * NU + j];
-          const float r = sigmoidf_acc(xr + ar);
-          const float z = sigmoidf_acc(xz + az);
-          const float nn = tanhf(xn + bin + r * an);
-          const float hnew = (1.f - z) * nn + z * hreg[m];
-          hreg[m] = hnew;
-          hbuf[(j >> 1) * RS + 2 * s + (j & 1)] = hnew;
-          const long long tb = s_tok[s];
-          if (tb >= 0) {
-            const long long tok = tb + (long long)t * prm.map.t_stride;
-            prm.out[(size_t)tok * (2 * NU) + d * NU + j] = hnew;
-            if (prm.stash) {
-              float* st4 = prm.stash + ((size_t)tok * 2 + d) * (4 * NU) + j;
-              st4[0] = r; st4[NU] = z; st4[2 * NU] = nn; st4[3 * NU] = an;
-            }
-          }
-        }
-      }
-    };
-
-    for (int step = 0; step < T; ++step) {
-      // phase 1: matmul of group A for this step | gates of group B for the previous step
-      matmul_A();
-      if (step > 0) finalize(step - 1, SA, S);
-      __syncthreads();
-      if (step > 0 && step + 1 < T) issue(step + 1);   // stage ((step-1) & 1) was consumed by the gates of B just above
-      // phase 2: matmul of group B | gates of group A, both for this step
-      matmul_B();
-      finalize(step, 0, SA);
-      __syncthreads();
-    }
-    finalize(T - 1, SA, S);
-  } else {
-    // few sequences per CTA (small batches): the step is pure latency, one phase pair per step is shorter
-    for (int step = 0; step < T; ++step) {
-      const int t = (d == 0) ? step : T - 1 - step;
-      const float* __restrict__ hc = s_h + (size_t)(step & 1) * (NU / 2) * RS;
-      float* __restrict__ hnx = s_h + (size_t)((step + 1) & 1) * (NU / 2) * RS;
-
-      // ---- partial products over this thread's slice of the previous hidden state, in passes of <= 6 sequences
-      //      (weights 60 + paired accumulators 36 + operands 12 registers stay under the 128-register budget)
-      {
-        const float* __restrict__ hp = hc + (size_t)(ig * IRP) * RS;
-        float* __restrict__ pp = s_part + (size_t)(ig * 3) * S * NU + j;
-        if constexpr (S == 16) {
-          fwd_partial_pass<NU, S, IRP, 0, 6>(w, hp, pp); fwd_partial_pass<NU, S, IRP, 6, 6>(w, hp, pp); fwd_partial_pass<NU, S, IRP, 12, 4>(w, hp, pp);
-        } else if constexpr (S == 14) {
-          fwd_partial_pass<NU, S, IRP, 0, 6>(w, hp, pp); fwd_partial_pass<NU, S, IRP, 6, 4>(w, hp, pp); fwd_partial_pass<NU, S, IRP, 10, 4>(w, hp, pp);
-        } else if constexpr (S == 12) {
-          fwd_partial_pass<NU, S, IRP, 0, 6>(w, hp, pp); fwd_partial_pass<NU, S, IRP, 6, 6>(w, hp, pp);
-        } else if constexpr (S == 8) {
-          fwd_partial_pass<NU, S, IRP, 0, 4>(w, hp, pp); fwd_partial_pass<NU, S, IRP, 4, 4>(w, hp, pp);
-        } else {
-          fwd_partial_pass<NU, S, IRP, 0, S>(w, hp, pp);
-        }
-      }
-      __syncthreads();
-
-      // ---- owner of (unit j, sequence s): combine partials, gate math, publish h
-      mbar_wait(&s_bar[step & 1], (step >> 1) & 1);
-      const float* __restrict__ gxs = s_gx + (size_t)(step & 1) * S * N3;
-  #pragma unroll
-      for (int m = 0; m < MI; ++m) {
-        const int s = ig + IG * m;
-        if (s < S) {
-          float ar = bhr, az = bhz, an = bhn;
-  #pragma unroll
-          for (int p = 0; p < IG; ++p) {
-            ar += s_part[((size_t)(p * 3 + 0) * S + s) * NU + j];
-            az += s_part[((size_t)(p * 3 + 1) * S + s) * NU + j];
-            an += s_part[((size_t)(p * 3 + 2) * S + s) * NU + j];
-          }
-          const float xr = gxs[s * N3 + j], xz = gxs[s * N3 + NU + j], xn = gxs[s * N3 + 2 * NU + j];
-          const float r = sigmoidf_acc(xr + ar);
-          const float z = sigmoidf_acc(xz + az);
-          const float nn = tanhf(xn + bin + r * an);
-          const float hnew = (1.f - z) * nn + z * hreg[m];
-          hreg[m] = hnew;
-          hnx[(j >> 1) * RS + 2 * s + (j & 1)] = hnew;
-          const long long tb = s_tok[s];
-          if (tb >= 0) {
-            const long long tok = tb + (long long)t * prm.map.t_stride;
-            prm.out[(size_t)tok * (2 * NU) + d * NU + j] = hnew;
-            if (prm.stash) {
-              float* st = prm.stash + ((size_t)tok * 2 + d) * (4 * NU) + j;
-              st[0] = r; st[NU] = z; st[2 * NU] = nn; st[3 * NU] = an;
-            }
-          }
-        }
-      }
-      __syncthreads();
-      if (step + 2 < T) issue(step + 2);  // stage (step & 1) was fully consumed before the barrier above
-    }
-  }
-}
-
-// one pass of the backward product over CN sequences: acc[u][s] = sum_k w{a,b}[k] . dg[k][C0+s] (pairs along g)
-template <int NU, int S, int GRP, int C0, int CN>
-__device__ __forceinline__ void bwd_partial_pass(const u64 (&wa)[GRP], const u64 (&wb)[GRP], const float* __restrict__ gp,
-                                                 float* __restrict__ pp) {
-  constexpr int RS = pair_row_stride(S);
-  u64 acc[2][CN];
-#pragma unroll
-  for (int s = 0; s < CN; ++s) { acc[0][s] = 0ull; acc[1][s] = 0ull; }
-#pragma unroll
-  for (int k = 0; k < GRP; ++k) {
-    u64 gv[CN];
-#pragma unroll
-    for (int c = 0; c < CN; c += 2) {
-      const ulonglong2 v = *reinterpret_cast<const ulonglong2*>(gp + k * RS + 2 * (C0 + c));
-      gv[c] = v.x; gv[c + 1] = v.y;
-    }
-#pragma unroll
-    for (int s = 0; s < CN; ++s) {
-      ffma2(acc[0][s], wa[k], gv[s]);
-      ffma2(acc[1][s], wb[k], gv[s]);
-    }
-  }
-#pragma unroll
-  for (int s = 0; s < CN; ++s) {
-    pp[(size_t)(C0 + s) * NU] = sum2(acc[0][s]);
-    pp[(size_t)(C0 + s) * NU + NU / 2] = sum2(acc[1][s]);
-  }
-}
-
-template <int NU, int S>
-struct RegBwdCfg {
-  static constexpr int GG = 8;                                  // groups along the gate dimension (3n)
-  static constexpr int GRP = (3 * NU + 2 * GG - 1) / (2 * GG);  // gate-row PAIRS per group (last group zero padded)
-  static constexpr int NT = (NU / 2) * GG;
-  static constexpr int IG = NT / NU;                            // owner groups for the elementwise phase
-  static constexpr int MI = (S + IG - 1) / IG;
-  static constexpr int STAGES = 2;
-  static constexpr int RS = pair_row_stride(S);
-  static constexpr int ROW = 6 * NU;                  // staged floats per (stage, sequence): stash 4n | h_prev n | dout n
-  static constexpr size_t in_floats = (size_t)STAGES * S * ROW;
-  static constexpr size_t dg_floats = (size_t)GG * GRP * RS;
-  static constexpr size_t part_floats = (size_t)GG * S * NU;
-  static constexpr size_t smem_bytes = (in_floats + dg_floats + part_floats) * sizeof(float) + 16 + 16 * 8;
-};
-
-template <int NU, int S>
-__global__ void __launch_bounds__(RegBwdCfg<NU, S>::NT, 1) gru_bwd_reg_kernel(const GruBwdParams prm) {
-  using Cfg = RegBwdCfg<NU, S>;
-  constexpr int GG = Cfg::GG, GRP = Cfg::GRP, IG = Cfg::IG, MI = Cfg::MI, N3 = 3 * NU, ROW = Cfg::ROW, HALF = NU / 2, RS = Cfg::RS;
-  static_assert(NU % 2 == 0 && Cfg::NT % NU == 0 && S <= 16 && S % 2 == 0, "unsupported shape");
-  extern __shared__ __align__(128) float smem[];
-  float* s_in = smem;                               // [STAGES][S][stash 4n | hprev n | dout n]
-  float* s_dg = s_in + Cfg::in_floats;              // [GG*GRP][RS]: element (g, s) at (g/2)*RS + 2 s + (g & 1)
-  float* s_part = s_dg + Cfg::dg_floats;            // [GG][S][n]
-  uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_part + Cfg::part_floats);
-  long long* s_tok = reinterpret_cast<long long*>(s_bar + 2);
-  const int d = blockIdx.y;
-  const int q0 = blockIdx.x * S;
-  const int T = prm.T;
-  const int tid = threadIdx.x;
-  const int n_valid = min(S, prm.n_seq - q0);
-  // matmul phase: thread = (unit pair p, gate-row group gg)
-  const int p = tid % HALF, gg = tid / HALF;
-  // elementwise phase: thread owns (unit j, sequences ig + IG*m)
-  const int j = tid % NU, ig = tid / NU;
-
-  if (tid == 0) {
-    mbar_init(&s_bar[0], 1);
-    mbar_init(&s_bar[1], 1);
-    fence_barrier_init();
-  }
-  for (int idx = tid; idx < (int)(Cfg::in_floats + Cfg::dg_floats); idx += Cfg::NT) smem[idx] = 0.f;
-
-  u64 wa[GRP], wb[GRP];
-  {
-    const float* __restrict__ wsrc = prm.w_hh + (size_t)d * N3 * NU;
-#pragma unroll
-    for (int k = 0; k < GRP; ++k) {
-      const int g = 2 * (gg * GRP + k);
-      const float a0 = g < N3 ? __ldg(wsrc + (size_t)g * NU + p) : 0.f;
-      const float a1 = g + 1 < N3 ? __ldg(wsrc + (size_t)(g + 1) * NU + p) : 0.f;
-      const float b0 = g < N3 ? __ldg(wsrc + (size_t)g * NU + p + HALF) : 0.f;
-      const float b1 = g + 1 < N3 ? __ldg(wsrc + (size_t)(g + 1) * NU + p + HALF) : 0.f;
-      wa[k] = pack2(a0, a1);
-      wb[k] = pack2(b0, b1);
-    }
-  }
-  float dhc[MI];
-#pragma unroll
-  for (int m = 0; m < MI; ++m) dhc[m] = 0.f;
-  if (tid < S) s_tok[tid] = tid < n_valid ? tok_base(prm.map, q0 + tid) : -1;
-  __syncthreads();
-  fence_proxy_async();
-
-  // producer: lane s of warp 0 fetches the three rows of sequence s for forward step `st`
-  auto issue = [&](int st, int slot) {
-    if (tid < 32) {
-      uint64_t* bar = &s_bar[slot];
-      const uint32_t per_seq = (st > 0 ? 6u : 5u) * NU * 4u;
-      if (tid == 0) mbar_arrive_expect_tx(bar, (uint32_t)n_valid * per_seq);
-      __syncwarp();
-      if (tid < n_valid) {
-        const int t = (d == 0) ? st : T - 1 - st;
-        const int tp = (d == 0) ? t - 1 : t + 1;
-        const long long b0 = s_tok[tid];
-        const long long tok = b0 + (long long)t * prm.map.t_stride;
-        float* dst = s_in + ((size_t)slot * S + tid) * ROW;
-        tma_bulk_g2s(dst, prm.stash + ((size_t)tok * 2 + d) * (4 * NU), 4u * NU * 4u, bar);
-        if (st > 0) {
-          const long long tokp = b0 + (long long)tp * prm.map.t_stride;
-          tma_bulk_g2s(dst + 4 * NU, prm.out + (size_t)tokp * (2 * NU) + d * NU, NU * 4u, bar);
-        }
-        tma_bulk_g2s(dst + 5 * NU, prm.dout + (size_t)tok * (2 * NU) + d * NU, NU * 4u, bar);
-      }
-    }
-  };
-  issue(T - 1, 0);
-  if (T > 1) issue(T - 2, 1);
-
-  int it = 0;
-  for (int step = T - 1; step >= 0; --step, ++it) {
-    const int t = (d == 0) ? step : T - 1 - step;
-    const int slot = it & 1;
-    mbar_wait(&s_bar[slot], (it >> 1) & 1);
-    const float* __restrict__ in = s_in + (size_t)slot * S * ROW;
-    float dhd[MI];
-#pragma unroll
-    for (int m = 0; m < MI; ++m) {
-      const int s = ig + IG * m;
-      dhd[m] = 0.f;
-      if (s < S) {
-        const float* row = in + (size_t)s * ROW;
-        const float r = row[j], z = row[NU + j], nn = row[2 * NU + j], hnn = row[3 * NU + j];
-        const float hprev = step > 0 ? row[4 * NU + j] : 0.f;
-        const float dh = row[5 * NU + j] + dhc[m];
-        const float dn = dh * (1.f - z);
-        const float dz = dh * (hprev - nn);
-        const float dn_pre = dn * (1.f - nn * nn);
-        const float dz_pre = dz * z * (1.f - z);
-        const float dr_pre = dn_pre * hnn * r * (1.f - r);
-        const float dnr = dn_pre * r;
-        dhd[m] = dh * z;
-        // NU is even, so gate row g = {0, n, 2n} + j has the parity of j
-        s_dg[(size_t)(j >> 1) * RS + 2 * s + (j & 1)] = dr_pre;
-        s_dg[(size_t)((NU + j) >> 1) * RS + 2 * s + (j & 1)] = dz_pre;
-        s_dg[(size_t)((2 * NU + j) >> 1) * RS + 2 * s + (j & 1)] = dnr;
-        const long long tb = s_tok[s];
-        if (tb >= 0) {
-          const long long tok = tb + (long long)t * prm.map.t_stride;
-          float* g = prm.dgx + ((size_t)tok * 2 + d) * N3 + j;
-          g[0] = dr_pre; g[NU] = dz_pre; g[2 * NU] = dn_pre;
-          prm.dghn[((size_t)tok * 2 + d) * NU + j] = dnr;
-        }
-      }
-    }
-    __syncthreads();                      // s_dg complete; stage `slot` fully consumed
-    if (step >= 2) issue(step - 2, slot);
-
-    // ---- dh_{step-1}[u] (+)= sum_g W_hh[g][u] * dg[g] over this thread's gate rows
-    {
-      const float* __restrict__ gp = s_dg + (size_t)(gg * GRP) * RS;
-      float* __restrict__ pp = s_part + (size_t)gg * S * NU + p;
-      if constexpr (S == 16) {
-        bwd_partial_pass<NU, S, GRP, 0, 6>(wa, wb, gp, pp); bwd_partial_pass<NU, S, GRP, 6, 6>(wa, wb, gp, pp); bwd_partial_pass<NU, S, GRP, 12, 4>(wa, wb, gp, pp);
-      } else if constexpr (S == 14) {
-        bwd_partial_pass<NU, S, GRP, 0, 6>(wa, wb, gp, pp); bwd_partial_pass<NU, S, GRP, 6, 4>(wa, wb, gp, pp); bwd_partial_pass<NU, S, GRP, 10, 4>(wa, wb, gp, pp);
-      } else if constexpr (S == 12) {
-        bwd_partial_pass<NU, S, GRP, 0, 6>(wa, wb, gp, pp); bwd_partial_pass<NU, S, GRP, 6, 6>(wa, wb, gp, pp);
-      } else if constexpr (S == 8) {
-        bwd_partial_pass<NU, S, GRP, 0, 4>(wa, wb, gp, pp); bwd_partial_pass<NU, S, GRP, 4, 4>(wa, wb, gp, pp);
-      } else {
-        bwd_partial_pass<NU, S, GRP, 0, S>(wa, wb, gp, pp);
-      }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int m = 0; m < MI; ++m) {
-      const int s = ig + IG * m;
-      if (s < S) {
-        float a = dhd[m];
-#pragma unroll
-        for (int q = 0; q < GG; ++q) a += s_part[((size_t)q * S + s) * NU + j];
-        dhc[m] = a;
-      }
-    }
-  }
-}
-
-
 // ================================================================================================ tensor-core scan
 // The recurrent product of a step, G[3n x S] = W_hh[3n x n] h[n x S], on the 5th-generation tensor cores:
 //   * W_hh lives in TENSOR MEMORY for the whole sweep as the A operand (one 128-row tile per gate, rows = hidden
@@ -749,7 +280,8 @@ __global__ void __launch_bounds__(RegBwdCfg<NU, S>::NT, 1) gru_bwd_reg_kernel(co
 //     registers, stores h / the stash rows (coalesced over j) and writes the next B operand;
 //   * the per-step gx rows arrive through a 3-stage TMA bulk-copy ring filled by a dedicated producer warp.
 // A step is ~1.5 k cycles of latency (MMA 0.5 k + gate math 0.7 k + hand-offs), below the ~2.3 k cycles the step's HBM
-// traffic costs at 148 CTAs, against 8.6 k cycles for the FFMA2 register kernel above.
+// traffic costs at 148 CTAs.  Keeping W_hh in registers with FFMA2 inner products instead was measured at 8.6 k cycles
+// per step (DESIGN.md).
 template <int NU>
 struct TcCfg {
   static constexpr int KP = (NU + 15) / 16 * 16;      // reduction length padded to the MMA's K = 16
@@ -1241,25 +773,9 @@ int launch_bwd_tc(const GruBwdParams& prm, int S, cudaStream_t stream) {
   return ISA_OK;
 }
 
-template <int NU, int S>
-int launch_fwd_reg(const GruFwdParams& prm, cudaStream_t stream) {
-  using Cfg = RegFwdCfg<NU, S>;
-  ISA_CUDA(cudaFuncSetAttribute(gru_fwd_reg_kernel<NU, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::smem_bytes));
-  dim3 grid((prm.n_seq + S - 1) / S, 2);
-  gru_fwd_reg_kernel<NU, S><<<grid, Cfg::NT, Cfg::smem_bytes, stream>>>(prm);
-  return ISA_OK;
-}
-template <int NU, int S>
-int launch_bwd_reg(const GruBwdParams& prm, cudaStream_t stream) {
-  using Cfg = RegBwdCfg<NU, S>;
-  ISA_CUDA(cudaFuncSetAttribute(gru_bwd_reg_kernel<NU, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::smem_bytes));
-  dim3 grid((prm.n_seq + S - 1) / S, 2);
-  gru_bwd_reg_kernel<NU, S><<<grid, Cfg::NT, Cfg::smem_bytes, stream>>>(prm);
-  return ISA_OK;
-}
-
-// sequences per CTA for the register-resident kernels: fewest waves over the SMs, then least work per step
-int pick_S_reg(int n_seq, int num_sms) {
+// sequences per CTA for the tensor-core kernels: fewest waves over the SMs, then least work per step
+// (S = 14 -> 148 CTAs for the 1024 rows of a batch-16 64x64 map, both directions)
+int pick_S_tc(int n_seq, int num_sms) {
   const int cand[5] = {16, 14, 12, 8, 4};
   int best = 4;
   long long best_cost = -1;
@@ -1310,20 +826,8 @@ int isa_gru_scan_fwd(const float* gx, const float* w_hh, const float* b_hh, cons
   prm.gx = gx; prm.w_hh = w_hh; prm.b_hh = b_hh; prm.b_ih = b_ih; prm.out = out; prm.stash = stash;
   prm.n_seq = n_seq; prm.T = T; prm.n = n_units;
   prm.map.inner = inner; prm.map.outer_stride = outer_tok_stride; prm.map.inner_stride = inner_tok_stride; prm.map.t_stride = t_tok_stride;
-  if (n_units == 100 && aligned16(gx) && !getenv("ISA_GRU_GENERIC") && !getenv("ISA_GRU_REG")) {
-    rc = launch_fwd_tc<100>(prm, pick_S_reg(n_seq, di.num_sms), stream);
-    if (rc) return rc;
-    ISA_CUDA(cudaGetLastError());
-    return ISA_OK;
-  }
-  if (n_units == 100 && aligned16(gx) && !getenv("ISA_GRU_GENERIC")) {
-    switch (pick_S_reg(n_seq, di.num_sms)) {
-      case 16: rc = launch_fwd_reg<100, 16>(prm, stream); break;
-      case 14: rc = launch_fwd_reg<100, 14>(prm, stream); break;
-      case 12: rc = launch_fwd_reg<100, 12>(prm, stream); break;
-      case 8: rc = launch_fwd_reg<100, 8>(prm, stream); break;
-      default: rc = launch_fwd_reg<100, 4>(prm, stream); break;
-    }
+  if (n_units == 100 && aligned16(gx)) {
+    rc = launch_fwd_tc<100>(prm, pick_S_tc(n_seq, di.num_sms), stream);
     if (rc) return rc;
     ISA_CUDA(cudaGetLastError());
     return ISA_OK;
@@ -1358,20 +862,8 @@ int isa_gru_scan_bwd(const float* dout, const float* out, const float* stash, co
   prm.dout = dout; prm.out = out; prm.stash = stash; prm.w_hh = w_hh; prm.dgx = dgx; prm.dghn = dghn;
   prm.n_seq = n_seq; prm.T = T; prm.n = n_units;
   prm.map.inner = inner; prm.map.outer_stride = outer_tok_stride; prm.map.inner_stride = inner_tok_stride; prm.map.t_stride = t_tok_stride;
-  if (n_units == 100 && aligned16(stash) && aligned16(out) && aligned16(dout) && !getenv("ISA_GRU_GENERIC") && !getenv("ISA_GRU_REG")) {
-    rc = launch_bwd_tc<100>(prm, pick_S_reg(n_seq, di.num_sms), stream);
-    if (rc) return rc;
-    ISA_CUDA(cudaGetLastError());
-    return ISA_OK;
-  }
-  if (n_units == 100 && aligned16(stash) && aligned16(out) && aligned16(dout) && !getenv("ISA_GRU_GENERIC")) {
-    switch (pick_S_reg(n_seq, di.num_sms)) {
-      case 16: rc = launch_bwd_reg<100, 16>(prm, stream); break;
-      case 14: rc = launch_bwd_reg<100, 14>(prm, stream); break;
-      case 12: rc = launch_bwd_reg<100, 12>(prm, stream); break;
-      case 8: rc = launch_bwd_reg<100, 8>(prm, stream); break;
-      default: rc = launch_bwd_reg<100, 4>(prm, stream); break;
-    }
+  if (n_units == 100 && aligned16(stash) && aligned16(out) && aligned16(dout)) {
+    rc = launch_bwd_tc<100>(prm, pick_S_tc(n_seq, di.num_sms), stream);
     if (rc) return rc;
     ISA_CUDA(cudaGetLastError());
     return ISA_OK;

@@ -24,7 +24,6 @@
 #include "isa_common.cuh"
 #include "isa_tcgen05.cuh"
 #include <math.h>
-#include <stdlib.h>
 
 namespace {
 
@@ -58,8 +57,6 @@ struct KmWs {
   int* state;              // [R] 0 active, 1 strict, 2 tol/max_iter
   int* n_iter;             // [R]
   long long* seed_pot;     // [k][R][kMaxL] potentials of the candidates of every k-means++ step (atomically summed)
-  unsigned* gen;           // [R] flow kernel: published Lloyd iteration of the restart | state << 24
-  unsigned* done;          // [R] flow kernel: slices that have finished their E-step, summed over the iterations
   unsigned long long* seed_prof;   // [6] CTA 0's phase times of the seeding kernel in ns: search, pass 1, pass 2, grid barriers; its search segments, rounds
   size_t zero_bytes;
   // not zeroed
@@ -108,8 +105,6 @@ KmWs km_carve(void* base, int ld, int C, int k, int R) {
   w.state = (int*)take(4 * (size_t)R);
   w.n_iter = (int*)take(4 * (size_t)R);
   w.seed_pot = (long long*)take(8 * (size_t)k * R * kMaxL);
-  w.gen = (unsigned*)take(4 * (size_t)R);
-  w.done = (unsigned*)take(4 * (size_t)R);
   w.seed_prof = (unsigned long long*)take(8 * 8);
   w.zero_bytes = off;
   w.mean = (float*)take(4 * (size_t)C);
@@ -162,17 +157,6 @@ __device__ __forceinline__ long long warp_sum_ll(long long v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
-}
-
-// 64-bit add on shared memory as two native 32-bit atomics (a 64-bit shared atomicAdd compiles to a CAS loop,
-// ATOMS.CAST.SPIN): every adder learns from the returned low word whether ITS addition wrapped and forwards
-// that carry, so the final value is exact once all adders are done (read it after a barrier).
-__device__ __forceinline__ void smem_add64(long long* addr, long long v) {
-  unsigned* p = reinterpret_cast<unsigned*>(addr);
-  const unsigned lo = (unsigned)(unsigned long long)v, hi = (unsigned)((unsigned long long)v >> 32);
-  const unsigned old = atomicAdd(p, lo);
-  const unsigned add_hi = hi + ((old + lo < old) ? 1u : 0u);
-  if (add_hi) atomicAdd(p + 1, add_hi);
 }
 
 __device__ __forceinline__ unsigned long long gtime_ns() {
@@ -826,9 +810,16 @@ struct LloydParams {
   double* inertia_out;  // [R]
   int* n_iter_out;      // [R]
   int* info;            // [16] status, best restart, n, total Lloyd iterations, then CTA 0's phase profile in us
-  int bounds;           // packed-FP32 kernel: Hamerly bounds (skip the points whose label provably cannot change) from this Lloyd iteration on, 0 = never
-  int priv;             // packed-FP32 kernel: accumulate the moved points of a CTA in shared memory (k*C int64 + k int)
 };
+
+// The packed-FP32 E-step with two points per thread skips, from this Lloyd iteration on, the points whose label provably
+// cannot change (Hamerly bounds).  Measured on one B200 box, same process order (Lloyd loop of the four benchmark images,
+// 49-52 k points, k = 16, 35 restarts, 3100-3700 restart-iterations): 9.73 / 9.59 / 11.18 / 8.71 ms without, 8.43 / 8.91 /
+// 10.50 / 8.20 ms with bounds from iteration 32 (80 % of the point visits skipped; what is left is the wait for the slowest
+// CTA, whose range holds the restarts that still move).  Planted clusters that converge in ~50 iterations: 9.26 -> 9.59 ms
+// (49 k points), 17.0 -> 17.5 ms (131 k): the bound arrays and the list passes cost 3 % there.  From iteration 1 / 6 / 16
+// the planted cases lose 10 / 8 / 4 % (loose bounds while every centre still moves) and the benchmark images gain no more.
+constexpr int kBoundsFrom = 32;
 
 typedef unsigned long long km_u64;
 __device__ __forceinline__ void km_ffma2(km_u64& acc, km_u64 a, km_u64 b) { asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc) : "l"(a), "l"(b)); }
@@ -921,64 +912,6 @@ __device__ __forceinline__ void estep_pair(const float* __restrict__ Xc, int ld,
     const float v0 = __fmaf_rn(-2.f, d0, cs), v1 = __fmaf_rn(-2.f, d1, cs);
     if (j == 0 || v0 < best[0]) { if (j) second[0] = best[0]; best[0] = v0; lab[0] = j; } else if (v0 < second[0]) second[0] = v0;
     if (j == 0 || v1 < best[1]) { if (j) second[1] = best[1]; best[1] = v1; lab[1] = j; } else if (v1 < second[1]) second[1] = v1;
-  }
-}
-
-// Scalar form for four points per thread: 4 centres x 4 points = 16 independent FFMA chains in the oracle's order and ONE
-// LDS.128 of plain centres per 16 FFMAs.  The packed form above needs a 16-byte {c, c} load per two FFMA2s: with four
-// schedulers sharing one LSU (512 B of register writes per warp-wide LDS.128 = 4 cycles) it is LSU bound at ~25 % of
-// the FP32 pipe; here the LSU and the FP32 pipe are balanced.
-template <int CP>
-__device__ __forceinline__ void estep_tile4(const float* __restrict__ Xc, int ld, int n, int C, int k, int tile,
-                                            const float* __restrict__ s_cent, const float* __restrict__ s_csq, int (&lab)[4]) {
-  constexpr int kTileP = kLloydThreads * 4;
-  const int base = tile * kTileP + threadIdx.x;
-  float x[4][CP];
-#pragma unroll
-  for (int p = 0; p < 4; ++p) {
-    const int i = base + p * kLloydThreads;
-#pragma unroll
-    for (int f = 0; f < CP; ++f) x[p][f] = (f < C && i < n) ? Xc[(size_t)f * ld + i] : 0.f;
-  }
-  float bv[4];
-#pragma unroll
-  for (int p = 0; p < 4; ++p) { bv[p] = 0.f; lab[p] = 0; }
-  for (int j0 = 0; j0 < k; j0 += 4) {
-    float acc[4][4];
-#pragma unroll
-    for (int p = 0; p < 4; ++p)
-#pragma unroll
-      for (int q = 0; q < 4; ++q) acc[p][q] = 0.f;
-#pragma unroll
-    for (int f4 = 0; f4 < CP; f4 += 4) {
-      float4 cv[4];
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        const int j = (j0 + q < k) ? j0 + q : k - 1;            // clamped: the extra results are discarded below
-        cv[q] = *reinterpret_cast<const float4*>(s_cent + (size_t)j * CP + f4);
-      }
-#pragma unroll
-      for (int q = 0; q < 4; ++q)
-#pragma unroll
-        for (int p = 0; p < 4; ++p) {
-          acc[p][q] = __fmaf_rn(x[p][f4 + 0], cv[q].x, acc[p][q]);
-          acc[p][q] = __fmaf_rn(x[p][f4 + 1], cv[q].y, acc[p][q]);
-          acc[p][q] = __fmaf_rn(x[p][f4 + 2], cv[q].z, acc[p][q]);
-          acc[p][q] = __fmaf_rn(x[p][f4 + 3], cv[q].w, acc[p][q]);
-        }
-    }
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      const int j = j0 + q;
-      if (j < k) {
-        const float cs = s_csq[j];
-#pragma unroll
-        for (int p = 0; p < 4; ++p) {
-          const float v = __fmaf_rn(-2.f, acc[p][q], cs);
-          if (j == 0 || v < bv[p]) { bv[p] = v; lab[p] = j; }
-        }
-      }
-    }
   }
 }
 
@@ -1172,8 +1105,6 @@ __global__ void __launch_bounds__(kLloydThreads, (PPT == 2 || TC) ? 2 : 1) km_ll
   float* s_csq = s_cent + k * CP;                                           // [k]
   float* s_cdup = s_csq + (k + 3) / 4 * 4;                                  // [k][CP] x {c, c} (16 B aligned); FFMA E-step only
   unsigned* s_moved = reinterpret_cast<unsigned*>(s_cdup + (TC ? 0 : (size_t)2 * k * CP));  // [kTile] (point in tile | old << 12 | new << 20)
-  long long* s_acc = reinterpret_cast<long long*>(s_moved + kMaxTile);          // [k][C] privatised centre-sum deltas (prm.priv)
-  int* s_acnt = reinterpret_cast<int*>(s_acc + (size_t)k * C);                  // [k] count deltas
   // tensor-core E-step: its own region behind the update's centres
   unsigned char* tc_base = smem_raw + (((size_t)(k * CP + (k + 3) / 4 * 4) * 4 + 127) / 128) * 128;
   const TcLayout tl = km_tc_layout(C, CP, k);
@@ -1212,28 +1143,9 @@ __global__ void __launch_bounds__(kLloydThreads, (PPT == 2 || TC) ? 2 : 1) km_ll
     // balanced contiguous ranges (sizes differ by at most one item; ceil-sized ranges left up to half the CTAs idle)
     const int it0 = (int)((long long)blockIdx.x * total / gridDim.x), it1 = (int)((long long)(blockIdx.x + 1) * total / gridDim.x);
     int cur = -1;
-    bool acc_dirty = false;
-    // privatised M-step (prm.priv): the exact fixed-point deltas of this CTA's moved points are summed in shared memory and
-    // reach the global sums once per (CTA, restart) -- k*C reductions instead of 2*C per moved point
-    auto flush_acc = [&](int r) {
-      __syncthreads();
-      long long* gs = ws.sums + (size_t)r * k * C;
-      int* gcnt = ws.cnt + (size_t)r * k;
-      for (int idx = threadIdx.x; idx < k * C; idx += kLloydThreads) {
-        const long long v = s_acc[idx];
-        if (v) { atomicAdd((unsigned long long*)(gs + idx), (unsigned long long)v); s_acc[idx] = 0; }
-      }
-      for (int j = threadIdx.x; j < k; j += kLloydThreads) {
-        const int c = s_acnt[j];
-        if (c) { atomicAdd(gcnt + j, c); s_acnt[j] = 0; }
-      }
-      __syncthreads();
-      acc_dirty = false;
-    };
     for (int item = it0; item < it1; ++item) {
       const int r = s_active[item / tiles], tile = item % tiles;
       if (r != cur) {
-        if (acc_dirty) flush_acc(cur);
         __syncthreads();
         load_centers(ws.centers + (size_t)r * k * C, s_cent, s_csq, k, C, CP, s_cdup);
         cur = r;
@@ -1251,8 +1163,7 @@ __global__ void __launch_bounds__(kLloydThreads, (PPT == 2 || TC) ? 2 : 1) km_ll
         aprev[p] = (i < n && mode == 0) ? acct[i] : 255;
       }
       int lab[kPPT];
-      if constexpr (PPT == 4 && CP <= 32) estep_tile4<CP>(Xc, ld, n, C, k, tile, s_cent, s_csq, lab);
-      else estep_tile<CP, PPT>(Xc, ld, n, C, k, tile, s_cdup, s_csq, lab);
+      estep_tile<CP, PPT>(Xc, ld, n, C, k, tile, s_cdup, s_csq, lab);
       bool any_changed = false;
 #pragma unroll
       for (int p = 0; p < kPPT; ++p) {
@@ -1284,21 +1195,8 @@ __global__ void __launch_bounds__(kLloydThreads, (PPT == 2 || TC) ? 2 : 1) km_ll
         const int nm = s_nmoved;
         long long* gs = ws.sums + (size_t)r * k * C;
         int* gcnt = ws.cnt + (size_t)r * k;
-        if (prm.priv && nm >= 8) {
-          acc_dirty = true;
-          for (int idx = threadIdx.x; idx < nm * C; idx += kLloydThreads) {
-            const int e = idx / C, f = idx - e * C;
-            const unsigned ent = s_moved[e];
-            const int li = ent & 0xfff, a = (ent >> 12) & 0xff, l = (ent >> 20) & 0xff;
-            const long long q = to_fixed(Xc[(size_t)f * ld + tile * kTile + li], sc.p_x);
-            if (a != 255) smem_add64(s_acc + a * C + f, -q);
-            smem_add64(s_acc + l * C + f, q);
-            if (f == 0) {
-              if (a != 255) atomicSub(s_acnt + a, 1);
-              atomicAdd(s_acnt + l, 1);
-            }
-          }
-        } else
+        // (the guard changes no result; without it ptxas spills in the 24-feature instance at 128 registers)
+        if (nm > 0)
         for (int idx = threadIdx.x; idx < nm * C; idx += kLloydThreads) {
           const int e = idx / C, f = idx - e * C;
           const unsigned ent = s_moved[e];
@@ -1313,7 +1211,6 @@ __global__ void __launch_bounds__(kLloydThreads, (PPT == 2 || TC) ? 2 : 1) km_ll
         }
       }
     }
-    if (acc_dirty) flush_acc(cur);
    }
   };
 
@@ -1771,10 +1668,6 @@ __global__ void __launch_bounds__(kLloydThreads, (PPT == 2 || TC) ? 2 : 1) km_ll
     __syncthreads();
   };
 
-  if (!TC && prm.priv) {
-    for (int idx = threadIdx.x; idx < k * C; idx += kLloydThreads) s_acc[idx] = 0;
-    for (int j = threadIdx.x; j < k; j += kLloydThreads) s_acnt[j] = 0;
-  }
   for (int idx = blockIdx.x * kLloydThreads + threadIdx.x; idx < R * k; idx += gridDim.x * kLloydThreads) ws.delta[idx] = 0.f;
   // labels / acct start as "none" (255)
   for (size_t idx = (size_t)blockIdx.x * kLloydThreads + threadIdx.x; idx < (size_t)R * ld; idx += (size_t)gridDim.x * kLloydThreads) {
@@ -1796,7 +1689,7 @@ __global__ void __launch_bounds__(kLloydThreads, (PPT == 2 || TC) ? 2 : 1) km_ll
     ++total_iters;
     // the bounds pay once most points have settled: the first iterations (nearly every point moves, the bounds are loose)
     // take the plain path; the first bounded iteration starts from U = inf and computes every point
-    if constexpr (TC) run_estep_tc(0); else if (PPT == 2 && prm.bounds && it >= prm.bounds) run_estep_bounds(0); else run_estep(0);
+    if constexpr (TC) run_estep_tc(0); else if (PPT == 2 && it >= kBoundsFrom) run_estep_bounds(0); else run_estep(0);
     lap(t_e);
     grid_barrier(ws.barrier, epoch);
     lap(t_b1);
@@ -1901,347 +1794,6 @@ __global__ void __launch_bounds__(kLloydThreads, (PPT == 2 || TC) ? 2 : 1) km_ll
 }
 
 
-// ------------------------------------------------------------------ Lloyd, dataflow variant (n <= 512 points per CTA)
-// The restarts are independent, so nothing needs a grid-wide barrier per iteration: every CTA owns ONE fixed slice of
-// the points for the whole kernel (its rows of X live in registers: no re-read per iteration) and processes that slice for
-// every restart whose next centres have been PUBLISHED (gen[r] = iteration | state << 24, release / acquire).  The CTA
-// that completes a restart's E-step (done[r] reaches slices x iteration) runs its centre update at once -- while the
-// other CTAs are busy with other restarts -- and publishes the next generation.  A restart that needs 250 iterations
-// no longer makes the other 34 pay a grid barrier, an update phase and a second barrier per iteration, and late in the
-// run (a few slow restarts left) an iteration costs its own ~10 us chain instead of ~60 us.  Arithmetic is unchanged
-// (same E-step fma order, same exact fixed-point sums, same update code): results stay bit-identical to the oracle.
-__device__ __forceinline__ void st_release_u32(unsigned* p, unsigned v) { asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
-
-constexpr int kFlowPPT = 4;                     // points per thread: one LDS.128 of a centre feeds 16 FFMAs
-constexpr int kFlowHalf = kLloydThreads / 2;    // the two halves of the CTA work on different restarts at the same time
-constexpr int kFlowSlice = kFlowHalf * kFlowPPT;   // 512 points per CTA at most
-
-template <int CP>
-__global__ void __launch_bounds__(kLloydThreads, 1) km_lloyd_flow_kernel(const LloydParams prm, int batch) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  const int n = *prm.n_ptr;
-  const int C = prm.C, k = prm.k, R = prm.R, ld = prm.ld;
-  const KmWs& ws = prm.ws;
-  const int status = *ws.status;
-  if (status) {
-    if (blockIdx.x == 0 && threadIdx.x < 16) prm.info[threadIdx.x] = threadIdx.x == 0 ? status : (threadIdx.x == 2 ? n : 0);
-    return;
-  }
-  // shared memory: [k][CP] scratch centres + [k] norms + {c, c} scratch (update / relocation), then per batch slot
-  // [k][CP] centres + norms, then the moved-point list of the whole batch
-  const int k4 = (k + 3) / 4 * 4;
-  float* s_cent = reinterpret_cast<float*>(smem_raw);                       // [k][CP]
-  float* s_csq = s_cent + k * CP;                                           // [k4]
-  float* s_centB = s_csq + k4;                                              // [batch][k][CP] (16 B aligned: k * CP % 4 == 0)
-  float* s_csqB = s_centB + (size_t)batch * k * CP;                         // [batch][k4]
-  unsigned* s_moved = reinterpret_cast<unsigned*>(s_csqB + (size_t)batch * k4);   // [batch * 512] (point | old << 9 | new << 17 | slot << 25)
-  __shared__ int s_nmoved;
-  __shared__ unsigned s_gen[kMaxInit], s_done[kMaxInit];
-  __shared__ int s_myiter[kMaxInit];
-  __shared__ unsigned char s_fin[kMaxInit];
-  __shared__ int s_ready[kMaxInit], s_final[kMaxInit], s_upd[kMaxInit], s_nready, s_nfinal, s_nupd;
-  __shared__ int s_chg[kMaxInit];
-  __shared__ long long s_redll[kLloydThreads / 32];
-
-  const KmScales sc = km_scales(*ws.maxabs_bits, n, C);
-  const float tol_abs = __double2float_rn(__dmul_rn(__ddiv_rn(__dmul_rn(__ll2double_rn(*ws.tolsum), sc.ip_t),
-                                                               __dmul_rn((double)n, (double)C)), prm.tol_rel));
-  const float* __restrict__ Xc = ws.Xc;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int half = threadIdx.x / kFlowHalf, th = threadIdx.x % kFlowHalf;
-  const int G = gridDim.x;
-  const int per = (((n + G - 1) / G) + 31) / 32 * 32;       // points per slice (<= 512: checked by the launcher through ld)
-  const int n_owner = (n + per - 1) / per;                  // CTAs with a non-empty slice
-  const int lo = blockIdx.x * per;
-  const int hi = min(n, lo + per);
-  const bool owner = lo < n;
-  unsigned epoch = 0;
-  const unsigned long long t_start = gtime_ns();
-
-  // this CTA's rows of X for the whole kernel: thread th of EITHER half holds points lo + th + 128 p, p = 0..3
-  float x[kFlowPPT][CP];
-  bool okp[kFlowPPT];
-#pragma unroll
-  for (int p = 0; p < kFlowPPT; ++p) {
-    const int i = lo + th + p * kFlowHalf;
-    okp[p] = i < hi;
-#pragma unroll
-    for (int f = 0; f < CP; ++f) x[p][f] = (f < C && okp[p]) ? Xc[(size_t)f * ld + i] : 0.f;
-  }
-  if (owner && half == 0)
-    for (int r = 0; r < R; ++r)
-#pragma unroll
-      for (int p = 0; p < kFlowPPT; ++p)
-        if (okp[p]) { ws.labels[(size_t)r * ld + lo + th + p * kFlowHalf] = 255; ws.acct[(size_t)r * ld + lo + th + p * kFlowHalf] = 255; }
-  for (int r = threadIdx.x; r < kMaxInit; r += kLloydThreads) { s_myiter[r] = 0; s_fin[r] = 0; }
-  __syncthreads();
-
-  // labels of this thread's four points against the centres in shared memory.  Scalar FFMAs in the oracle's order (feature
-  // ascending per (point, centre)); 4 centres x 4 points = 16 independent chains, one LDS.128 per 16 FFMAs (the packed
-  // FFMA2 form of the barrier kernel needs a 16-byte {c, c} load per TWO instructions and is bound by the LSU at ~25 %).
-  auto estep = [&](const float* __restrict__ cent, const float* __restrict__ csq, int (&lab)[kFlowPPT]) {
-    float bv[kFlowPPT];
-#pragma unroll
-    for (int p = 0; p < kFlowPPT; ++p) { bv[p] = 0.f; lab[p] = 0; }
-    for (int j0 = 0; j0 < k; j0 += 4) {
-      float acc[kFlowPPT][4];
-#pragma unroll
-      for (int p = 0; p < kFlowPPT; ++p)
-#pragma unroll
-        for (int q = 0; q < 4; ++q) acc[p][q] = 0.f;
-#pragma unroll
-      for (int f4 = 0; f4 < CP; f4 += 4) {
-        float4 cv[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          const int j = (j0 + q < k) ? j0 + q : k - 1;            // clamped: the extra results are discarded below
-          cv[q] = *reinterpret_cast<const float4*>(cent + (size_t)j * CP + f4);
-        }
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-#pragma unroll
-          for (int p = 0; p < kFlowPPT; ++p) {
-            acc[p][q] = __fmaf_rn(x[p][f4 + 0], cv[q].x, acc[p][q]);
-            acc[p][q] = __fmaf_rn(x[p][f4 + 1], cv[q].y, acc[p][q]);
-            acc[p][q] = __fmaf_rn(x[p][f4 + 2], cv[q].z, acc[p][q]);
-            acc[p][q] = __fmaf_rn(x[p][f4 + 3], cv[q].w, acc[p][q]);
-          }
-      }
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        const int j = j0 + q;
-        if (j < k) {
-          const float cs = csq[j];
-#pragma unroll
-          for (int p = 0; p < kFlowPPT; ++p) {
-            const float v = __fmaf_rn(-2.f, acc[p][q], cs);
-            if (j == 0 || v < bv[p]) { bv[p] = v; lab[p] = j; }
-          }
-        }
-      }
-    }
-  };
-
-  // CTA 0's phase profile (ns): polling / idle, centre updates, centre loads, E-steps, M-step moves + fence, final passes
-  unsigned long long t_poll = 0, t_upd = 0, t_ld = 0, t_e = 0, t_m = 0, t_f = 0, t_mark = gtime_ns();
-  auto lap = [&](unsigned long long& acc) { const unsigned long long t = gtime_ns(); acc += t - t_mark; t_mark = t; };
-  int rounds = 0;
-  if (owner) {
-    int n_fin = 0;
-    while (n_fin < R) {
-      if (threadIdx.x < R) {                                   // one L2 round trip for all restarts
-        s_gen[threadIdx.x] = ld_acquire_u32(ws.gen + threadIdx.x);
-        s_done[threadIdx.x] = ld_acquire_u32(ws.done + threadIdx.x);
-      }
-      __syncthreads();
-      if (threadIdx.x == 0) {
-        int nr = 0, nf = 0, nu = 0;
-        for (int r = 0; r < R; ++r) {
-          if (s_fin[r]) continue;
-          const unsigned g = s_gen[r];
-          const int it = (int)(g & 0xffffffu);
-          if (g >> 24) s_final[nf++] = r;                                        // converged: final labels + inertia
-          else if (it == s_myiter[r] && nr < batch) s_ready[nr++] = r;           // next centres are published
-          // the centre update of restart r belongs to slice r % n_owner: due once every slice has added its E-step
-          else if (r % n_owner == (int)blockIdx.x && it + 1 == s_myiter[r] && s_done[r] == (unsigned)n_owner * (unsigned)(it + 1))
-            s_upd[nu++] = r;
-        }
-        s_nready = nr; s_nfinal = nf; s_nupd = nu; s_nmoved = 0;
-      }
-      for (int b = threadIdx.x; b < kMaxInit; b += kLloydThreads) s_chg[b] = 0;
-      __syncthreads();
-      const int nready = s_nready, nfinal = s_nfinal, nupd = s_nupd;
-      if (nready == 0 && nfinal == 0 && nupd == 0) { __nanosleep(100); __syncthreads(); lap(t_poll); continue; }
-      lap(t_poll);
-      ++rounds;
-      // ---- centre updates this slice is responsible for (the other slices run theirs at the same time)
-      for (int u = 0; u < nupd; ++u) {
-        const int r = s_upd[u];
-        const int it = s_myiter[r] - 1;
-        __threadfence();                                       // acquire: the other slices' sums / labels, no stale L1 lines
-        lloyd_update_restart<CP>(prm, sc, tol_abs, r, it, n, s_cent, s_csq);
-        __threadfence();
-        __syncthreads();
-        if (threadIdx.x == 0) st_release_u32(ws.gen + r, (unsigned)(it + 1) | ((unsigned)__ldcg(ws.state + r) << 24));
-        __syncthreads();
-      }
-      lap(t_upd);
-      // ---- centres of every ready restart -> shared memory (zero padded to CP) + norms
-      if (C == CP) {
-        const int v4 = k * CP / 4;
-        for (int idx = threadIdx.x; idx < nready * v4; idx += kLloydThreads) {
-          const int b = idx / v4, e = idx - b * v4;
-          reinterpret_cast<float4*>(s_centB + (size_t)b * k * CP)[e] = __ldcg(reinterpret_cast<const float4*>(ws.centers + (size_t)s_ready[b] * k * C) + e);
-        }
-      } else {
-        for (int idx = threadIdx.x; idx < nready * k * CP; idx += kLloydThreads) {
-          const int b = idx / (k * CP), rem = idx - b * (k * CP), j = rem / CP, f = rem - j * CP;
-          s_centB[(size_t)b * k * CP + rem] = (f < C) ? __ldcg(ws.centers + ((size_t)s_ready[b] * k + j) * C + f) : 0.f;
-        }
-      }
-      __syncthreads();
-      for (int idx = threadIdx.x; idx < nready * k; idx += kLloydThreads) {
-        const int b = idx / k, j = idx - b * k;
-        const float* c = s_centB + ((size_t)b * k + j) * CP;
-        float a = 0.f;
-        for (int f = 0; f < C; ++f) a = __fmaf_rn(c[f], c[f], a);
-        s_csqB[b * k4 + j] = a;
-      }
-      __syncthreads();
-      lap(t_ld);
-
-      // ---- E-steps of the batch, two restarts at a time (one per half of the CTA, no CTA barrier inside)
-      for (int b = half; b < nready; b += 2) {
-        const int r = s_ready[b];
-        unsigned char* labels = ws.labels + (size_t)r * ld + lo + th;
-        unsigned char* acct = ws.acct + (size_t)r * ld + lo + th;
-        int lp[kFlowPPT], ap[kFlowPPT];
-#pragma unroll
-        for (int p = 0; p < kFlowPPT; ++p) {
-          lp[p] = okp[p] ? (int)labels[p * kFlowHalf] : 0;
-          // acct can be rewritten by another CTA (empty-cluster relocation in the update): never from L1
-          ap[p] = okp[p] ? (int)__ldcg(acct + p * kFlowHalf) : 255;
-        }
-        int lab[kFlowPPT];
-        estep(s_centB + (size_t)b * k * CP, s_csqB + b * k4, lab);
-        bool any_changed = false;
-#pragma unroll
-        for (int p = 0; p < kFlowPPT; ++p) {
-          bool moved = false;
-          if (okp[p]) {
-            moved = (lab[p] != ap[p]);
-            if (moved) acct[p * kFlowHalf] = (unsigned char)lab[p];
-            if (lab[p] != lp[p]) { labels[p * kFlowHalf] = (unsigned char)lab[p]; any_changed = true; }
-          }
-          const unsigned bal = __ballot_sync(0xffffffffu, moved);
-          if (bal) {
-            int base = 0;
-            if (lane == 0) base = atomicAdd(&s_nmoved, __popc(bal));
-            base = __shfl_sync(0xffffffffu, base, 0);
-            if (moved) s_moved[base + __popc(bal & ((1u << lane) - 1u))] =
-                (unsigned)(th + p * kFlowHalf) | ((unsigned)ap[p] << 9) | ((unsigned)lab[p] << 17) | ((unsigned)b << 25);
-          }
-        }
-        if (__any_sync(0xffffffffu, any_changed) && lane == 0) s_chg[b] = 1;
-      }
-      __syncthreads();
-      lap(t_e);
-      // ---- incremental M-step of the batch: exact fixed-point moves with native 64-bit reductions
-      {
-        const int nm = s_nmoved;
-        for (int idx = threadIdx.x; idx < nm * C; idx += kLloydThreads) {
-          const int e = idx / C, f = idx - e * C;
-          const unsigned ent = s_moved[e];
-          const int li = ent & 0x1ff, a = (ent >> 9) & 0xff, l = (ent >> 17) & 0xff, b = ent >> 25;
-          const int r = s_ready[b];
-          long long* gs = ws.sums + (size_t)r * k * C;
-          int* gcnt = ws.cnt + (size_t)r * k;
-          const long long q = to_fixed(Xc[(size_t)f * ld + lo + li], sc.p_x);
-          if (a != 255) atomicAdd((unsigned long long*)(gs + a * C + f), (unsigned long long)(-q));
-          atomicAdd((unsigned long long*)(gs + l * C + f), (unsigned long long)q);
-          if (f == 0) {
-            if (a != 255) atomicSub(gcnt + a, 1);
-            atomicAdd(gcnt + l, 1);
-          }
-        }
-        if (threadIdx.x < nready && s_chg[threadIdx.x]) ws.changed[s_ready[threadIdx.x]] = 1;
-      }
-      // ---- completion: one fence, then one counter increment per restart of the batch (in parallel)
-      __threadfence();
-      __syncthreads();
-      if (threadIdx.x < nready) {
-        const int r = s_ready[threadIdx.x];
-        s_myiter[r] += 1;
-        atomicAdd(ws.done + r, 1u);
-      }
-      __syncthreads();
-      lap(t_m);
-      // ---- converged restarts: final labels (re-run of the E-step unless strict) and this slice's inertia
-      for (int q = 0; q < nfinal; ++q) {
-        const int r = s_final[q];
-        const int st = (int)(s_gen[r] >> 24);
-        unsigned char* labels = ws.labels + (size_t)r * ld + lo + th;
-        __syncthreads();
-        load_centers(ws.centers + (size_t)r * k * C, s_cent, s_csq, k, C, CP);
-        long long acc = 0;
-        if (half == 0) {
-          int lab[kFlowPPT];
-          if (st == 2) {
-            estep(s_cent, s_csq, lab);
-#pragma unroll
-            for (int p = 0; p < kFlowPPT; ++p)
-              if (okp[p]) labels[p * kFlowHalf] = (unsigned char)lab[p];
-          } else {
-#pragma unroll
-            for (int p = 0; p < kFlowPPT; ++p) lab[p] = okp[p] ? (int)labels[p * kFlowHalf] : 0;
-          }
-#pragma unroll
-          for (int p = 0; p < kFlowPPT; ++p) {
-            const float* c = s_cent + lab[p] * CP;
-            float d = 0.f;
-#pragma unroll
-            for (int f = 0; f < CP; ++f)
-              if (f < C) { const float t = __fsub_rn(x[p][f], c[f]); d = __fmaf_rn(t, t, d); }
-            if (okp[p]) acc += to_fixed(d, sc.p_d);
-          }
-        }
-        acc = warp_sum_ll(acc);
-        if (lane == 0) s_redll[warp] = acc;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-          long long t = 0;
-          for (int w = 0; w < kLloydThreads / 32; ++w) t += s_redll[w];
-          if (t) atomicAdd((unsigned long long*)(ws.inertia_q + r), (unsigned long long)t);
-          s_fin[r] = 1;
-        }
-        ++n_fin;
-      }
-      __syncthreads();      // every thread is done with this snapshot before the next one overwrites it
-      lap(t_f);
-    }
-  }
-  grid_barrier(ws.barrier, epoch);
-  const unsigned long long t_loop_end = gtime_ns();
-
-  // ---- best restart: lowest inertia unless it is the same clustering (KMeans.fit, _kmeans.py:1534-1541)
-  if (blockIdx.x == 0) {
-    __shared__ int s_mapmin[256], s_mapmax[256];
-    int best = 0;
-    int max_it = 0;
-    for (int r = 0; r < R; ++r) max_it = max(max_it, __ldcg(ws.n_iter + r));
-    for (int r = 1; r < R; ++r) {
-      if (__ldcg(ws.inertia_q + r) < __ldcg(ws.inertia_q + best)) {
-        for (int j = threadIdx.x; j < 256; j += kLloydThreads) { s_mapmin[j] = 0x7fffffff; s_mapmax[j] = -1; }
-        __syncthreads();
-        const unsigned char* l1 = ws.labels + (size_t)r * ld;
-        const unsigned char* l2 = ws.labels + (size_t)best * ld;
-        for (int i = threadIdx.x; i < n; i += kLloydThreads) {
-          const int a = l1[i], b = l2[i];
-          if (s_mapmin[a] > b) atomicMin(&s_mapmin[a], b);
-          if (s_mapmax[a] < b) atomicMax(&s_mapmax[a], b);
-        }
-        __syncthreads();
-        const int bad = __syncthreads_or(threadIdx.x < 256 && s_mapmax[threadIdx.x] >= 0 && s_mapmin[threadIdx.x] != s_mapmax[threadIdx.x]);
-        if (bad) best = r;  // not the same clustering -> take the better restart
-      }
-    }
-    const unsigned char* lb = ws.labels + (size_t)best * ld;
-    for (int i = threadIdx.x; i < n; i += kLloydThreads) prm.labels_out[i] = lb[i];
-    for (int idx = threadIdx.x; idx < k * C; idx += kLloydThreads)
-      prm.centers_out[idx] = __fadd_rn(__ldcg(ws.centers + (size_t)best * k * C + idx), ws.mean[idx % C]);
-    for (int r = threadIdx.x; r < R; r += kLloydThreads) {
-      prm.inertia_out[r] = __dmul_rn(__ll2double_rn(__ldcg(ws.inertia_q + r)), sc.ip_d);
-      prm.n_iter_out[r] = __ldcg(ws.n_iter + r);
-    }
-    if (threadIdx.x == 0) {
-      prm.info[0] = 0; prm.info[1] = best; prm.info[2] = n; prm.info[3] = max_it;
-      prm.info[4] = (int)(t_e / 1000); prm.info[5] = (int)(t_poll / 1000); prm.info[6] = (int)(t_upd / 1000); prm.info[7] = (int)(t_m / 1000);
-      prm.info[8] = (int)((t_loop_end - t_start) / 1000); prm.info[9] = (int)((gtime_ns() - t_loop_end) / 1000);
-      prm.info[10] = (int)(t_ld / 1000); prm.info[11] = (int)(t_f / 1000); prm.info[12] = rounds;
-    }
-  }
-}
-
 size_t lloyd_smem_bytes(int k, int C, int CP) {
   size_t fl = (size_t)3 * k * CP + (k + 3) / 4 * 4;
   return fl * 4 + (size_t)kMaxTile * 4 + 16;
@@ -2289,8 +1841,7 @@ int launch_seed_v(const int* n_ptr, int ld, int C, int k, int L, int R, const do
 template <int CP>
 int launch_seed(const int* n_ptr, int ld, int C, int k, int L, int R, const double* uniforms, const KmWs& ws, int num_sms, cudaStream_t stream) {
   bool launched = false;
-  int rc = ISA_OK;
-  if (!getenv("ISA_KM_STREAMING")) rc = launch_seed_v<CP, true>(n_ptr, ld, C, k, L, R, uniforms, ws, num_sms, stream, &launched);
+  const int rc = launch_seed_v<CP, true>(n_ptr, ld, C, k, L, R, uniforms, ws, num_sms, stream, &launched);
   if (rc || launched) return rc;
   return launch_seed_v<CP, false>(n_ptr, ld, C, k, L, R, uniforms, ws, num_sms, stream, &launched);
 }
@@ -2317,23 +1868,8 @@ int launch_lloyd_tc(const LloydParams& prm, int num_sms, cudaStream_t stream) {
 }
 
 template <int CP, int PPT>
-int launch_lloyd_ppt(const LloydParams& prm_in, int num_sms, cudaStream_t stream) {
-  LloydParams prm = prm_in;
-  size_t smem = lloyd_smem_bytes(prm.k, prm.C, CP);
-  const size_t extra = (size_t)prm.k * prm.C * 8 + (size_t)(prm.k + 3) / 4 * 4 * 4 + 16;
-  // Measured on B200 (49 k points, C = 24, k = 16, 35 restarts): E-phase 5.99 ms with the shared-memory accumulation against
-  // 6.06 ms with direct RED.64s -- the reductions are not what the E-phase waits for; kept behind ISA_KM_PRIV=1.
-  prm.priv = (getenv("ISA_KM_PRIV") && (smem + extra) * 2 <= 200 * 1024) ? 1 : 0;   // must not cost the second CTA per SM
-  if (prm.priv) smem += extra;
-  // bounds from Lloyd iteration prm.bounds on (0 = never); ISA_KM_BOUNDS_FROM=<it> / ISA_KM_NOBOUNDS=1 for experiments.
-  // Measured on one B200 box, same process order (Lloyd loop of the four benchmark images, 49-52 k points, k = 16, 35
-  // restarts, 3100-3700 restart-iterations): 9.73 / 9.59 / 11.18 / 8.71 ms without, 8.43 / 8.91 / 10.50 / 8.20 ms with bounds
-  // from iteration 32 (80 % of the point visits skipped; what is left is the wait for the slowest CTA, whose range
-  // holds the restarts that still move).  Planted clusters that converge in ~50 iterations: 9.26 -> 9.59 ms (49 k points),
-  // 17.0 -> 17.5 ms (131 k): the bound arrays and the list passes cost 3 % there.  From iteration 1 / 6 / 16 the planted
-  // cases lose 10 / 8 / 4 % (loose bounds while every centre still moves) and the benchmark images gain no more.
-  prm.bounds = (PPT == 2 && !getenv("ISA_KM_NOBOUNDS")) ? (getenv("ISA_KM_BOUNDS_FROM") ? atoi(getenv("ISA_KM_BOUNDS_FROM")) : 32) : 0;
-  if (prm.bounds < 0) prm.bounds = 0;
+int launch_lloyd_ppt(const LloydParams& prm, int num_sms, cudaStream_t stream) {
+  const size_t smem = lloyd_smem_bytes(prm.k, prm.C, CP);
   const void* fn = (const void*)km_lloyd_kernel<CP, PPT, false>;
   ISA_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   // static + dynamic may exceed 48 KB
   int occ = 0;
@@ -2345,59 +1881,17 @@ int launch_lloyd_ppt(const LloydParams& prm_in, int num_sms, cudaStream_t stream
   return ISA_OK;
 }
 
-// 2 points per thread and two CTAs per SM (one CTA's loads overlap the other's distance loop) unless the embedding
-// is too wide for 128 registers; ISA_KM_PPT=2|4 overrides (experiments).
-template <int CP>
-int launch_lloyd_flow(const LloydParams& prm, int num_sms, int max_smem, cudaStream_t stream, bool* launched) {
-  *launched = false;
-  const int k = prm.k, k4 = (k + 3) / 4 * 4;
-  const size_t fixed = ((size_t)k * CP + k4) * 4 + 64;
-  const size_t per_slot = (size_t)k * CP * 4 + (size_t)k4 * 4 + kFlowSlice * 4;
-  const size_t budget = (size_t)max_smem > 8192 ? (size_t)max_smem - 8192 : 0;     // static shared memory + margin
-  if (budget < fixed + per_slot) return ISA_OK;
-  int batch = (int)((budget - fixed) / per_slot);
-  if (batch > prm.R) batch = prm.R;
-  if (batch > 63) batch = 63;                                                       // 6-bit slot field of the moved list
-  const size_t smem = fixed + (size_t)batch * per_slot;
-  const void* fn = (const void*)km_lloyd_flow_kernel<CP>;
-  if (smem > 48 * 1024) ISA_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int occ = 0;
-  ISA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, kLloydThreads, smem));
-  if (occ < 1) return ISA_OK;
-  void* args[] = {(void*)&prm, (void*)&batch};
-  ISA_CUDA(cudaLaunchCooperativeKernel(fn, dim3(num_sms), dim3(kLloydThreads), args, smem, stream));
-  *launched = true;
-  return ISA_OK;
-}
-
 template <int CP>
 int launch_lloyd(const LloydParams& prm, int num_sms, cudaStream_t stream) {
-  // Few enough points for one resident slice per SM: the barrier-free dataflow kernel is available behind ISA_KM_FLOW=1.
-  // Measured on B200 (49 k points, C = 24, k = 16, 35 restarts, 8934 restart-iterations): 28.0 ms against 21.2 ms for the
-  // barrier kernel below -- its E-step runs at the same ~46 % of the FP32 pipe (one LDS.128 per 16 FFMAs is the LSU's
-  // break-even: 512 B of register writes per warp-wide load) and the polling rounds (6.3 ms) cost more than the two grid
-  // barriers per iteration they replace (4.1 ms).  Kept as the measured alternative, not the default.
-  if ((long long)prm.ld <= 480LL * num_sms && CP <= 32 && getenv("ISA_KM_FLOW")) {
-    bool launched = false;
-    IsaDeviceInfo di;
-    int rc = isa_device_info(&di);
-    if (rc) return rc;
-    rc = launch_lloyd_flow<CP>(prm, num_sms, di.max_smem_optin, stream, &launched);
-    if (rc || launched) return rc;
-  }
-  // default: the tensor-core E-step (ISA_KM_FFMA=1 keeps the packed-FP32 kernel: the measured alternative and the
-  // path for C > 32 or k > 128)
-  // Measured on B200 (tools/bench_kmeans.py): k = 64, C = 32, 524 k points: 114 ms against 135 ms for the packed-FP32
-  // kernel (E-steps 60 / 80 ms); k = 16, C = 24: 10.3 against 8.9 ms (49 k points), 19.2 against 16.7 ms (131 k): with 16
-  // centres the per-item costs of the batch (operand conversion, MMA round trip, tensor-memory reads, the exact pass)
-  // outweigh the 384 FFMAs per point they replace.  Default: tensor cores from 33 centres on; ISA_KM_TC=1 / ISA_KM_FFMA=1 force.
-  const bool want_tc = getenv("ISA_KM_TC") ? true : (getenv("ISA_KM_FFMA") ? false : prm.k > 32);
-  if (CP <= 32 && km_tc_ok(prm.C, prm.k) && want_tc) return launch_lloyd_tc<CP>(prm, num_sms, stream);
-  int ppt = (CP <= 32) ? 2 : 4;   // ISA_KM_PPT=4 with CP <= 32 selects the scalar four-point E-step (estep_tile4): same speed
-  const char* e = getenv("ISA_KM_PPT");
-  if (e && (e[0] == '2' || e[0] == '4')) ppt = e[0] - '0';
-  if (ppt == 2) return launch_lloyd_ppt<CP, 2>(prm, num_sms, stream);
-  return launch_lloyd_ppt<CP, 4>(prm, num_sms, stream);
+  // Tensor-core E-step from 33 centres on.  Measured on B200 (tools/bench_kmeans.py): k = 64, C = 32, 524 k points: 114 ms
+  // against 135 ms for the packed-FP32 kernel (E-steps 60 / 80 ms); k = 16, C = 24: 10.3 against 8.9 ms (49 k points),
+  // 19.2 against 16.7 ms (131 k): with 16 centres the per-item costs of the batch (operand conversion, MMA round trip,
+  // tensor-memory reads, the exact pass) outweigh the 384 FFMAs per point they replace.
+  if (CP <= 32 && km_tc_ok(prm.C, prm.k) && prm.k > 32) return launch_lloyd_tc<CP>(prm, num_sms, stream);
+  // packed FP32: 2 points per thread and two CTAs per SM (one CTA's loads overlap the other's distance loop) unless the
+  // embedding is too wide for 128 registers
+  if constexpr (CP <= 32) return launch_lloyd_ppt<CP, 2>(prm, num_sms, stream);
+  else return launch_lloyd_ppt<CP, 4>(prm, num_sms, stream);
 }
 
 int pick_cp(int C) { return C <= 8 ? 8 : C <= 16 ? 16 : C <= 24 ? 24 : C <= 32 ? 32 : 64; }
@@ -2458,7 +1952,7 @@ int isa_kmeans_fit(const float* X, const int* n_ptr, int ld, int C, int k, int n
   LloydParams prm;
   prm.n_ptr = n_ptr; prm.ld = ld; prm.C = C; prm.k = k; prm.R = n_init; prm.max_iter = max_iter; prm.tol_rel = tol_rel;
   prm.ws = ws; prm.labels_out = labels_out; prm.centers_out = centers_out; prm.inertia_out = inertia_out;
-  prm.n_iter_out = n_iter_out; prm.info = info; prm.priv = 0; prm.bounds = 0;
+  prm.n_iter_out = n_iter_out; prm.info = info;
   switch (CP) {
     case 8: rc = launch_lloyd<8>(prm, di.num_sms, stream); break;
     case 16: rc = launch_lloyd<16>(prm, di.num_sms, stream); break;

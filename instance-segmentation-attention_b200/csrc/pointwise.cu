@@ -12,7 +12,6 @@
 #include "isa_common.cuh"
 #include "isa_ptx.cuh"
 #include "isa_tcgen05.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -1190,7 +1189,7 @@ int isa_pixel_heads_fwd(const float* xa, int Ca, const float* xb, int Cb, const 
   const int Co = Co0 + Co1, cop = (Co + 3) & ~3;
   const long long n_tiles = (P + kHeadTile - 1) / kHeadTile;
   long long grid = n_tiles < (long long)di.num_sms * 3 ? n_tiles : (long long)di.num_sms * 3;
-  if (Ca + Cb <= kHtKP && !getenv("ISA_HEADS_FFMA")) {
+  if (Ca + Cb <= kHtKP) {
     // tensor-core path: 2 CTAs per SM (256 TMEM columns each)
     size_t smem = 2 * kHtWPart + (size_t)kHeadTile * (Ca + Cb) * sizeof(float) + 64 + 128;
     if (smem < 80 * 1024) smem = 80 * 1024;     // never three CTAs on one SM: the third would spin in tcgen05.alloc
@@ -1233,7 +1232,7 @@ int isa_pixel_heads_bwd(const float* g0, int Co0, const float* g1, int Co1, cons
   const long long n_tiles = (P + kHeadTile - 1) / kHeadTile;
   long long grid = n_tiles < (long long)di.num_sms * 3 ? n_tiles : (long long)di.num_sms * 3;
   const int Kp = (Ca + Cb + 3) & ~3;
-  if (Ca + Cb <= kHtKP && !getenv("ISA_HEADS_FFMA")) {
+  if (Ca + Cb <= kHtKP) {
     size_t smem = 2 * kHbWPart + (size_t)kHeadTile * (Ca + Cb) * sizeof(float) + 64 + 128;
     if (smem < 80 * 1024) smem = 80 * 1024;     // at most two CTAs per SM (256 TMEM columns each)
     grid = n_tiles < (long long)di.num_sms * 2 ? n_tiles : (long long)di.num_sms * 2;
@@ -1287,7 +1286,7 @@ int isa_pixel_heads_wgrad(const float* g0, int Co0, const float* g1, int Co1, co
   const long long n_tiles = (P + kWgTile - 1) / kWgTile;
   const int grid = (int)(n_tiles < (long long)di.num_sms * 2 ? n_tiles : (long long)di.num_sms * 2);
   float* partial = reinterpret_cast<float*>(workspace);
-  if (K + 1 <= kHtKP && !getenv("ISA_HEADS_FFMA")) {
+  if (K + 1 <= kHtKP) {
     size_t smem = 2 * kHtWPart + (size_t)kHeadTile * K * sizeof(float) + 64 + 128;
     if (smem < 80 * 1024) smem = 80 * 1024;     // at most two CTAs per SM (256 TMEM columns each)
     const long long nt = (P + kHeadTile - 1) / kHeadTile;

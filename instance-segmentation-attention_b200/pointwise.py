@@ -13,8 +13,6 @@
         weight gradient (out x in = 24 x 24 from 65 536 rows) is a split-K batched GEMM instead of the single-CTA
         SIMT sgemm the library picks for that shape.
 """
-import os
-
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
@@ -121,7 +119,7 @@ class ConvBiasAct(nn.Conv2d):
     def forward(self, x):
         if (self.relu and self.bias is not None and x.is_cuda and x.dtype == torch.float32 and self.padding_mode == 'zeros'
                 and not isinstance(self.padding, str) and self.weight.shape[0] <= 256
-                and x.is_contiguous(memory_format=torch.channels_last) and os.environ.get("ISA_CONV_EPILOGUE") != "kernel"):
+                and x.is_contiguous(memory_format=torch.channels_last)):
             return _ConvBiasReluFn.apply(x, self.weight, self.bias, tuple(self.stride), tuple(self.padding), tuple(self.dilation), self.groups)
         y = self._conv_forward(x, self.weight, None)
         if self.bias is None:

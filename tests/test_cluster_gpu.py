@@ -64,24 +64,24 @@ def test_network_embeddings_bit_exact_and_sklearn_golden(cuda, golden_dir, case)
     assert KM.same_up_to_permutation(labels, g[name + "_sk_labels"])
 
 
-@pytest.mark.parametrize("env", ["ISA_KM_TC=1", "ISA_KM_NOBOUNDS=1", "ISA_KM_BOUNDS_FROM=1", "ISA_KM_BOUNDS_FROM=3", "ISA_KM_PRIV=1",
-                                 "ISA_KM_STREAMING=1"])
-def test_every_lloyd_variant_is_bit_exact(cuda, monkeypatch, env):
-    """The measured alternatives behind the environment switches (tensor-core filter at k = 16, no bounds, bounds from the
-    first iterations, privatised M-step, streaming seeding) all reproduce the oracle bit for bit on a near-tied network
-    embedding and on a planted case with few points per centre."""
-    key, val = env.split("=")
-    monkeypatch.setenv(key, val)
-    X = net_inputs("net0")
-    o = KM.kmeans_oracle(X, 16, seed=0, n_init=8)
-    labels, res = _gpu_fit(cuda, X, 16, seed=0, n_init=8)
-    _assert_same_as_oracle(labels, res, o)
+def _planted_3001():
     rs = np.random.RandomState(1)
     cent = rs.standard_normal((20, 12)) * 2
-    Y = (cent[rs.randint(0, 20, 3001)] + rs.standard_normal((3001, 12))).astype(np.float32)
-    o = KM.kmeans_oracle(Y, 40, seed=4, n_init=5)
-    labels, res = _gpu_fit(cuda, Y, 40, seed=4, n_init=5)
+    return (cent[rs.randint(0, 20, 3001)] + rs.standard_normal((3001, 12))).astype(np.float32)
+
+
+@pytest.mark.parametrize("data,k,n_init,seed", [("net0", 16, 8, 0), ("net0", 40, 4, 0), ("planted", 40, 5, 4)],
+                         ids=["net0_k16_packed_fp32", "net0_k40_tensor_core", "planted_k40_tensor_core"])
+def test_lloyd_paths_bit_exact(cuda, data, k, n_init, seed):
+    """The Lloyd E-step paths, each reached through its input, reproduce the oracle bit for bit: the packed-FP32 kernel
+    with the Hamerly bounds on a near-tied network embedding (k = 16), the tensor-core filter on the same embedding
+    (k = 40) and on a planted case with few points per centre (k = 40, C = 12)."""
+    X = net_inputs("net0") if data == "net0" else _planted_3001()
+    o = KM.kmeans_oracle(X, k, seed=seed, n_init=n_init)
+    labels, res = _gpu_fit(cuda, X, k, seed=seed, n_init=n_init)
     _assert_same_as_oracle(labels, res, o)
+    if k <= 32:
+        assert int(res.n_iter.max()) > 32, "the bounded E-step (from Lloyd iteration 32 on) never ran"
 
 
 def test_cumsum_search_edge_cases(cuda):

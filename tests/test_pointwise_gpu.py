@@ -52,25 +52,20 @@ def test_conv_modules_match_stock_layers(cuda):
         torch.testing.assert_close(ours.bias.grad, ref.bias.grad, rtol=1e-4, atol=1e-3)
 
 
-def test_conv_epilogue_in_cudnn_equals_epilogue_kernel(cuda, monkeypatch):
-    """relu(conv + bias) with the epilogue inside cuDNN's convolution (default) against the bias-free convolution followed
-    by the in-place epilogue kernel (ISA_CONV_EPILOGUE=kernel): same output bit for bit, same gradients."""
-    from isa_b200.pointwise import ConvBiasAct
+def test_conv_epilogue_in_cudnn_equals_epilogue_kernel(cuda):
+    """relu(conv + bias) with the epilogue inside cuDNN's convolution (ConvBiasAct) against the bias-free convolution
+    followed by the in-place epilogue kernel: same output bit for bit, same gradients."""
+    from isa_b200.pointwise import ConvBiasAct, bias_act_
     torch.manual_seed(5)
     m = ConvBiasAct(16, 32, 3, padding=1, relu=True).to(cuda)
     x = torch.randn(3, 16, 40, 28, device=cuda).contiguous(memory_format=torch.channels_last)
     g = torch.randn(3, 32, 40, 28, device=cuda).contiguous(memory_format=torch.channels_last)
     outs = []
-    for mode in (None, "kernel"):
-        if mode:
-            monkeypatch.setenv("ISA_CONV_EPILOGUE", mode)
-        else:
-            monkeypatch.delenv("ISA_CONV_EPILOGUE", raising=False)
-        m.zero_grad()
+    for fused in (True, False):
         xa = x.clone().requires_grad_(True)
-        y = m(xa)
-        y.backward(g)
-        outs.append((y.detach().clone(), xa.grad.clone(), m.weight.grad.clone(), m.bias.grad.clone()))
+        y = m(xa) if fused else bias_act_(F.conv2d(xa, m.weight, None, padding=1), m.bias, True)
+        grads = torch.autograd.grad(y, (xa, m.weight, m.bias), g)
+        outs.append((y.detach(),) + grads)
     assert torch.equal(outs[0][0], outs[1][0])
     for a, b in zip(outs[0][1:], outs[1][1:]):
         torch.testing.assert_close(a, b, rtol=1e-4, atol=1e-4)
@@ -117,7 +112,9 @@ def test_thin_linear_matches_linear(cuda, rows, cin, cout):
         torch.testing.assert_close(a, b, rtol=1e-4, atol=2e-3)
 
 
-@pytest.mark.parametrize("n,Ca,Cb,H,W,Co0,Co1", [(2, 50, 64, 32, 40, 2, 24), (1, 6, 2, 9, 7, 3, 5), (3, 50, 64, 16, 16, 2, 0), (1, 20, 12, 8, 8, 2, 30)])
+# (2, 80, 64, ...): more than 128 source channels, so forward, input gradient and weight gradient run the FFMA kernels
+@pytest.mark.parametrize("n,Ca,Cb,H,W,Co0,Co1", [(2, 50, 64, 32, 40, 2, 24), (1, 6, 2, 9, 7, 3, 5), (3, 50, 64, 16, 16, 2, 0), (1, 20, 12, 8, 8, 2, 30),
+                                                 (2, 80, 64, 16, 16, 2, 24)])
 def test_pixel_heads_match_conv_of_concatenation(cuda, n, Ca, Cb, H, W, Co0, Co1):
     from isa_b200.pointwise import pixel_heads
     torch.manual_seed(Ca + Cb + Co1)

@@ -35,7 +35,7 @@ def main():
     it_sum = int(res.n_iter.sum())
     out = {"n": n, "C": C, "k": k, "n_init": n_init, "ms_median": float(np.median(ts[1:])), "ms_min": float(np.min(ts)),
            "lloyd_iters_total": it_sum, "lloyd_iters_max": int(res.n_iter.max()), "grid_iters": int(res.info[3])}
-    out["lloyd_phase_us(estep,bar1|poll,update,bar2|mstep,loop,tail,[flow: centre loads, final passes, rounds])"] = [int(v) for v in res.info[4:13].cpu()]
+    out["lloyd_phase_us(estep,bar1,update,bar2,loop,tail)"] = [int(v) for v in res.info[4:10].cpu()]
     med = out["ms_median"] * 1e-3
     out["restart_iters_per_s"] = it_sum / med
     out["GFMA_per_s"] = it_sum * n * k * C / med / 1e9
