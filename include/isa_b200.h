@@ -193,7 +193,10 @@ int isa_attention_bwd(const float* q, const float* k, const float* v, const floa
  * (n_seq=B*W, T=H, inner=W, H*W, 1, W).  h_0 = 0.  n_units: multiple of 4, <= 128.
  * Backward writes dgx [tokens][2][3n] (gradient of the input projection; its r,z thirds are also the
  * hidden-side gate gradients) and dghn [tokens][2][n] (hidden-side n-gate gradient r*dn_pre);
- * weight/bias gradients are GEMMs / column sums over those (done by the caller). */
+ * weight/bias gradients are GEMMs / column sums over those (done by the caller).
+ * Pointers need only fp32 (4-byte) alignment.  n_units = 100 with a 16-byte-aligned gx selects the tensor-core
+ * forward, and n_units = 100 with 16-byte-aligned stash, out and dout the tensor-core backward; every other call runs
+ * the generic kernels, which compute the same recurrence. */
 int isa_gru_scan_fwd(const float* gx, const float* w_hh, const float* b_hh, const float* b_ih, int n_seq, int T, int n_units,
                      int inner, long long outer_tok_stride, long long inner_tok_stride, long long t_tok_stride,
                      float* out, float* stash, isa_stream_t stream);

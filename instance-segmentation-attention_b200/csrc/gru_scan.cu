@@ -361,8 +361,9 @@ __global__ void __launch_bounds__(TcCfg<NU>::NT, 1) gru_fwd_tc_kernel(const GruF
           const int k = c * 16 + 2 * e;
           float a = 0.f, b = 0.f;
           if (j < NU && k < NU) {          // NU even: k and k + 1 are valid together
-            const float2 v = __ldg(reinterpret_cast<const float2*>(wsrc + (size_t)(g * NU + j) * NU + k));
-            a = v.x; b = v.y;
+            // two scalar loads: the C-ABI promises w_hh only fp32 alignment, so a float2 load could be misaligned
+            const float* p = wsrc + (size_t)(g * NU + j) * NU + k;
+            a = __ldg(p); b = __ldg(p + 1);
           }
           split2(a, b, hi[e], lo[e]);
         }
