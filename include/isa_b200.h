@@ -62,6 +62,11 @@ int isa_selftest_grid_barrier(int ctas_per_sm, int threads, int iters, int varia
  * if some pixel is not one-hot (soft / overlapping masks) the kernels keep reading the dense masks.
  * workspace  isa_disc_loss_workspace_bytes(bs,C,K,H,W) bytes; hand the SAME buffer, untouched,
  *            to isa_disc_loss_bwd (it carries the per-instance sums saved for backward).
+ * Limits: 1 <= bs <= 65535, 1 <= C <= 64, 1 <= K <= 254, H*W < 2^30, norm 1 or 2 (else ISA_ERR_BAD_ARG).
+ * The column-walk forward keeps 4 * (K*(CP+1) + K*(2C+1) + 256*((C+1)|1)) bytes in shared memory (CP = C rounded up to
+ * 8, 16, 24, 32 or 64).  It runs for every dense target, and for a label map whose bs is above the label-map kernel's
+ * co-resident CTAs.  Where that does not fit an SM those calls return ISA_ERR_UNSUPPORTED; on a B200 (232,448 B of
+ * shared memory per CTA) that is C >= 54 with K above a bound that falls from 252 at C = 54 to 213 at C = 64.  Every call is checked before anything is enqueued: a refused call leaves every buffer as it was.
  */
 #define ISA_TGT_LABEL_U8 0
 #define ISA_TGT_DENSE_F32 1
@@ -69,6 +74,20 @@ int isa_selftest_grid_barrier(int ctas_per_sm, int threads, int iters, int varia
 #define ISA_TGT_DENSE_U8 3
 
 size_t isa_disc_loss_workspace_bytes(int bs, int C, int K, int H, int W);
+
+/* What isa_disc_loss_fwd / isa_disc_loss_bwd launch for these sizes on the current device; enqueues nothing.
+ * h_plan [ISA_DISC_PLAN_LEN] host ints:
+ *   0 route (ISA_DISC_ROUTE_*), 1 CP (padded channel count of the kernels' templates),
+ *   2 priv of the label-map kernel (1: per-warp accumulators, bit-reproducible; 0: one CTA accumulator with shared
+ *     atomics; -1: the route has no label-map kernel), 3 its CTAs per image, 4 its grid, 5 its dynamic shared memory (bytes),
+ *   6 CTAs per image of the column walk (0 when the route has none), 7 its grid, 8 its dynamic shared memory,
+ *   9 dynamic shared memory of the backward's prep kernel, 10 the backward's CTAs per image, 11 its dynamic shared memory.
+ * Returns ISA_ERR_BAD_ARG as the forward does, and ISA_ERR_UNSUPPORTED when no route fits. */
+#define ISA_DISC_ROUTE_LAB 0           /* label map: the label-map kernel alone */
+#define ISA_DISC_ROUTE_COL_THEN_LAB 1  /* dense target: the column walk (which returns at once if the masks are one-hot), then the label-map kernel */
+#define ISA_DISC_ROUTE_COL 2           /* the column walk alone (on a dense one-hot target: on the label map distilled from it) */
+#define ISA_DISC_PLAN_LEN 12
+int isa_disc_loss_plan(int target_kind, int bs, int C, int K, int H, int W, int* h_plan);
 
 int isa_disc_loss_fwd(const float* emb, const void* target, int target_kind, const int* n_objects,
                       int bs, int C, int H, int W, int K,

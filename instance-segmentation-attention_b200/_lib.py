@@ -32,6 +32,7 @@ SIGNATURES = {
     "isa_selftest_grid_barrier": (c_int, [c_int, c_int, c_int, c_int, c_void_p, ctypes.POINTER(c_float)]),
     # discriminative loss
     "isa_disc_loss_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
+    "isa_disc_loss_plan": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_int)]),
     "isa_disc_loss_fwd": (c_int, [c_void_p, c_void_p, c_int, c_void_p,
                                   c_int, c_int, c_int, c_int, c_int,
                                   c_float, c_float, c_int, c_int,

@@ -33,6 +33,7 @@
 namespace {
 
 enum { TGT_LABEL_U8 = 0, TGT_DENSE_F32 = 1, TGT_DENSE_I64 = 2, TGT_DENSE_U8 = 3 };
+enum { ROUTE_LAB = 0, ROUTE_COL_THEN_LAB = 1, ROUTE_COL = 2 };   // ISA_DISC_ROUTE_* of include/isa_b200.h
 
 constexpr int kThreads = 256;
 constexpr int kWarps = kThreads / 32;
@@ -1080,33 +1081,6 @@ int allow_smem(const void* fn, size_t smem) {
 }
 
 template <int CP>
-int launch_fwd(const FwdParams& prm, int grid, size_t smem, cudaStream_t stream) {
-  void* args[] = {(void*)&prm};
-  const void* fn = nullptr;
-  switch (prm.target_kind) {
-    case TGT_LABEL_U8: fn = (const void*)disc_fwd_kernel<CP, TGT_LABEL_U8>; break;
-    case TGT_DENSE_F32: fn = (const void*)disc_fwd_kernel<CP, TGT_DENSE_F32>; break;
-    case TGT_DENSE_I64: fn = (const void*)disc_fwd_kernel<CP, TGT_DENSE_I64>; break;
-    default: fn = (const void*)disc_fwd_kernel<CP, TGT_DENSE_U8>; break;
-  }
-  ISA_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, smem, stream));
-  return ISA_OK;
-}
-template <int CP>
-int occupancy_fwd(int kind, size_t smem, int* out) {
-  const void* fn = nullptr;
-  switch (kind) {
-    case TGT_LABEL_U8: fn = (const void*)disc_fwd_kernel<CP, TGT_LABEL_U8>; break;
-    case TGT_DENSE_F32: fn = (const void*)disc_fwd_kernel<CP, TGT_DENSE_F32>; break;
-    case TGT_DENSE_I64: fn = (const void*)disc_fwd_kernel<CP, TGT_DENSE_I64>; break;
-    default: fn = (const void*)disc_fwd_kernel<CP, TGT_DENSE_U8>; break;
-  }
-  int rc = allow_smem(fn, smem);
-  if (rc) return rc;
-  ISA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(out, fn, kThreads, smem));
-  return ISA_OK;
-}
-template <int CP>
 int launch_bwd(const BwdParams& prm, dim3 grid, size_t smem, cudaStream_t stream) {
   if (smem > 48 * 1024) {
     int rc = 0;
@@ -1152,6 +1126,136 @@ int check_common(int target_kind, int bs, int C, int H, int W, int K, int norm) 
   return ISA_OK;
 }
 
+const void* lab_kernel_fn(int CP) {
+  switch (CP) {
+    case 8: return (const void*)disc_fwd_lab_kernel<8>;
+    case 16: return (const void*)disc_fwd_lab_kernel<16>;
+    case 24: return (const void*)disc_fwd_lab_kernel<24>;
+    case 32: return (const void*)disc_fwd_lab_kernel<32>;
+    default: return (const void*)disc_fwd_lab_kernel<64>;
+  }
+}
+
+template <int CP>
+const void* col_kernel_fn_cp(int kind) {
+  switch (kind) {
+    case TGT_LABEL_U8: return (const void*)disc_fwd_kernel<CP, TGT_LABEL_U8>;
+    case TGT_DENSE_F32: return (const void*)disc_fwd_kernel<CP, TGT_DENSE_F32>;
+    case TGT_DENSE_I64: return (const void*)disc_fwd_kernel<CP, TGT_DENSE_I64>;
+    default: return (const void*)disc_fwd_kernel<CP, TGT_DENSE_U8>;
+  }
+}
+const void* col_kernel_fn(int CP, int kind) {
+  switch (CP) {
+    case 8: return col_kernel_fn_cp<8>(kind);
+    case 16: return col_kernel_fn_cp<16>(kind);
+    case 24: return col_kernel_fn_cp<24>(kind);
+    case 32: return col_kernel_fn_cp<32>(kind);
+    default: return col_kernel_fn_cp<64>(kind);
+  }
+}
+
+// Whether `fn` can take `smem` bytes of dynamic shared memory on top of its static ones; if so, opts it in.
+int smem_fits(const void* fn, size_t smem, const IsaDeviceInfo& di, bool* fits) {
+  cudaFuncAttributes fa;
+  ISA_CUDA(cudaFuncGetAttributes(&fa, fn));
+  *fits = smem + fa.sharedSizeBytes <= (size_t)di.max_smem_optin;
+  return *fits ? allow_smem(fn, smem) : ISA_OK;
+}
+
+// What isa_disc_loss_fwd / isa_disc_loss_bwd launch (see isa_disc_loss_plan).  Decided on the host from the sizes and
+// the device alone, before anything is enqueued, so that a refused call leaves every buffer untouched.
+struct DiscPlan {
+  int route;                 // ISA_DISC_ROUTE_*; -1 when only the backward was planned
+  int CP;
+  int priv, lab_G, lab_grid; // label-map kernel
+  size_t lab_smem;
+  int col_G, col_grid;       // column walk
+  int strips, rowsplits, rpt;
+  size_t col_smem;
+  size_t prep_smem;          // backward: disc_bwd_prep_kernel, then disc_bwd_kernel on a (bwd_gx, bs) grid
+  int bwd_gx;
+  size_t bwd_smem;
+};
+
+int make_plan(int target_kind, int bs, int C, int K, int H, int W, bool fwd, const IsaDeviceInfo& di, DiscPlan* pl) {
+  DiscPlan& p = *pl;
+  const int P = H * W;
+  p = DiscPlan{};
+  p.route = -1;
+  p.CP = pick_cp(C);
+  p.priv = -1;
+
+  // ---- backward: the prep kernel's [K][C] Gamma and the streaming kernel's mu and T in shared memory
+  ISA_CHECK_ARG(bs <= 65535, "disc_loss: bs=%d > 65535", bs);
+  p.prep_smem = sizeof(float) * (size_t)K * C;
+  p.bwd_smem = sizeof(float) * 2 * (size_t)K * (p.CP + 1);
+  int gx = (P + kThreads - 1) / kThreads;
+  const int per_img = (di.num_sms * 8 + bs - 1) / bs;
+  if (gx > per_img) gx = per_img;
+  p.bwd_gx = gx < 1 ? 1 : gx;
+  bool fits = false;
+  int rc = smem_fits((const void*)disc_bwd_prep_kernel, p.prep_smem, di, &fits);
+  if (rc) return rc;
+  if (!fits) { isa_set_error("disc_loss_bwd: prep kernel needs %zu B of shared memory", p.prep_smem); return ISA_ERR_UNSUPPORTED; }
+  if (!fwd) return ISA_OK;
+
+  // ---- label-map forward (one grid barrier, deterministic): label maps, and dense masks that turn out one-hot
+  const size_t acc1 = sizeof(float) * (size_t)K * (C + 1), mu = sizeof(float) * (size_t)K * (p.CP + 1);
+  const int priv = (mu + kWarps * acc1 <= 100 * 1024) ? 1 : 0;
+  const size_t lab_smem = mu + (priv ? kWarps : 1) * acc1;
+  const void* lab_fn = lab_kernel_fn(p.CP);
+  bool use_lab = false;
+  rc = smem_fits(lab_fn, lab_smem, di, &fits);
+  if (rc) return rc;
+  if (fits) {
+    int occ = 0;
+    ISA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, lab_fn, kThreads, lab_smem));
+    if (occ > 2) occ = 2;
+    int nbc = di.num_sms * occ;
+    if (nbc > kLabMaxCtas) nbc = kLabMaxCtas;
+    if (occ >= 1 && bs <= nbc) {
+      use_lab = true;
+      int G = nbc / bs;
+      const int maxG = (P + 255) / 256;          // no point in CTAs with fewer than one warp-round of pixels
+      if (G > maxG) G = maxG;
+      if (G < 1) G = 1;
+      p.priv = priv;
+      p.lab_G = G;
+      p.lab_grid = G * bs;
+      p.lab_smem = lab_smem;
+    }
+  }
+  if (use_lab && target_kind == TGT_LABEL_U8) { p.route = ROUTE_LAB; return ISA_OK; }
+
+  // ---- column-walk forward: soft / overlapping dense masks (and the fallback when the label-map kernel does not fit).
+  // On a dense target it always runs first: it finds out whether the masks are one-hot.
+  const size_t smem = sizeof(float) * ((size_t)K * (p.CP + 1) + (size_t)K * (2 * C + 1) + (size_t)kWarps * 32 * ((C + 1) | 1));
+  const void* col_fn = col_kernel_fn(p.CP, target_kind);
+  rc = smem_fits(col_fn, smem, di, &fits);
+  if (rc) return rc;
+  int occ = 0;
+  if (fits) ISA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, col_fn, kThreads, smem));
+  if (occ < 1) {
+    isa_set_error("disc_loss_fwd: the column-walk kernel needs %zu B of shared memory at C=%d K=%d (more than an SM has); it runs "
+                  "for every dense target and for label maps with bs=%d above the co-resident CTAs", smem, C, K, bs);
+    return ISA_ERR_UNSUPPORTED;
+  }
+  const int NB = di.num_sms * occ;  // co-resident CTAs
+  int G, grid;
+  if (bs <= NB) { G = NB / bs; grid = G * bs; } else { G = 1; grid = NB; }
+  p.col_G = G;
+  p.col_grid = grid;
+  p.col_smem = smem;
+  p.strips = (W + 31) / 32;
+  int rowsplits = (G * kWarps) / p.strips;
+  rowsplits = rowsplits < 1 ? 1 : (rowsplits > H ? H : rowsplits);
+  p.rpt = (H + rowsplits - 1) / rowsplits;
+  p.rowsplits = (H + p.rpt - 1) / p.rpt;
+  p.route = use_lab ? ROUTE_COL_THEN_LAB : ROUTE_COL;
+  return ISA_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1159,6 +1263,23 @@ extern "C" {
 size_t isa_disc_loss_workspace_bytes(int bs, int C, int K, int H, int W) {
   if (bs <= 0 || C <= 0 || K <= 0 || H <= 0 || W <= 0) return 0;
   return carve(nullptr, bs, C, K, H * W).total_bytes;
+}
+
+int isa_disc_loss_plan(int target_kind, int bs, int C, int K, int H, int W, int* h_plan) {
+  int rc = check_common(target_kind, bs, C, H, W, K, 2);
+  if (rc) return rc;
+  ISA_CHECK_ARG(h_plan, "disc_loss_plan: null pointer");
+  IsaDeviceInfo di;
+  rc = isa_device_info(&di);
+  if (rc) return rc;
+  DiscPlan pl;
+  rc = make_plan(target_kind, bs, C, K, H, W, true, di, &pl);
+  if (rc) return rc;
+  const int v[] = {pl.route, pl.CP, pl.priv, pl.lab_G, pl.lab_grid, (int)pl.lab_smem, pl.col_G, pl.col_grid, (int)pl.col_smem,
+                   (int)pl.prep_smem, pl.bwd_gx, (int)pl.bwd_smem};
+  static_assert(sizeof(v) / sizeof(v[0]) == 12, "ISA_DISC_PLAN_LEN");
+  for (int i = 0; i < 12; ++i) h_plan[i] = v[i];
+  return ISA_OK;
 }
 
 int isa_disc_loss_fwd(const float* emb, const void* target, int target_kind, const int* n_objects,
@@ -1185,103 +1306,30 @@ int isa_disc_loss_fwd(const float* emb, const void* target, int target_kind, con
   prm.w_var = w_var; prm.w_dist = w_dist; prm.w_reg = w_reg; prm.w_q = w_q;
   prm.out_loss = out_loss; prm.out_terms = out_terms; prm.out_means = out_means; prm.q_den = q_den;
 
-  const int CP = pick_cp(C);
+  DiscPlan pl;
+  rc = make_plan(target_kind, bs, C, K, H, W, true, di, &pl);
+  if (rc) return rc;
+
   ISA_CUDA(cudaMemsetAsync(workspace, 0, prm.ws.zero_bytes, stream));
   if (target_kind != TGT_LABEL_U8) {
     rc = launch_onehot_to_labels(target, target_kind, bs, K, H * W, prm.ws.labels, prm.ws.not_onehot, di.num_sms, stream);
     if (rc) return rc;
   }
-
-  // ---- label-map forward (one grid barrier, deterministic): label maps, and dense masks that turn out one-hot
-  LabParams lp;
-  bool use_lab = true;
-  size_t lab_smem = 0;
-  int lab_grid = 0;
-  if (use_lab) {
-    const size_t acc1 = sizeof(float) * (size_t)K * (C + 1), mu = sizeof(float) * (size_t)K * (CP + 1);
-    lp.priv = (mu + kWarps * acc1 <= 100 * 1024) ? 1 : 0;
-    lab_smem = mu + (lp.priv ? kWarps : 1) * acc1;
-    const void* fn = nullptr;
-    switch (CP) {
-      case 8: fn = (const void*)disc_fwd_lab_kernel<8>; break;
-      case 16: fn = (const void*)disc_fwd_lab_kernel<16>; break;
-      case 24: fn = (const void*)disc_fwd_lab_kernel<24>; break;
-      case 32: fn = (const void*)disc_fwd_lab_kernel<32>; break;
-      default: fn = (const void*)disc_fwd_lab_kernel<64>; break;
-    }
-    if (lab_smem > (size_t)di.max_smem_optin) use_lab = false;
-    int occ = 0;
-    if (use_lab) {
-      rc = allow_smem(fn, lab_smem);
-      if (rc) return rc;
-      ISA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, kThreads, lab_smem));
-      if (occ > 2) occ = 2;
-      int nbc = di.num_sms * occ;
-      if (nbc > kLabMaxCtas) nbc = kLabMaxCtas;
-      if (occ < 1 || bs > nbc) use_lab = false;
-      else {
-        const int P = H * W;
-        int G = nbc / bs;
-        const int maxG = (P + 255) / 256;          // no point in CTAs with fewer than one warp-round of pixels
-        if (G > maxG) G = maxG;
-        if (G < 1) G = 1;
-        lp.G = G;
-        lp.chunk = (((P + G - 1) / G) + 31) / 32 * 32;
-        lab_grid = G * bs;
-      }
-    }
-    if (use_lab) {
-      lp.f = prm;
-      lp.f.G = 1; lp.f.strips = 0; lp.f.rowsplits = 0; lp.f.rpt = 0; lp.f.lab_kernel_follows = 0;
-      if (target_kind == TGT_LABEL_U8) {
-        void* args[] = {(void*)&lp};
-        ISA_CUDA(cudaLaunchCooperativeKernel(fn, dim3(lab_grid), dim3(kThreads), args, lab_smem, stream));
-        return ISA_OK;
-      }
-    }
+  if (pl.route != ROUTE_LAB) {
+    prm.G = pl.col_G; prm.strips = pl.strips; prm.rowsplits = pl.rowsplits; prm.rpt = pl.rpt;
+    prm.lab_kernel_follows = (pl.route == ROUTE_COL_THEN_LAB) ? 1 : 0;
+    void* args[] = {(void*)&prm};
+    ISA_CUDA(cudaLaunchCooperativeKernel(col_kernel_fn(pl.CP, target_kind), dim3(pl.col_grid), dim3(kThreads), args, pl.col_smem, stream));
   }
-
-  // ---- column-walk forward: soft / overlapping dense masks (and the fallback when the label-map kernel does not fit)
-  const size_t smem = sizeof(float) * ((size_t)K * (CP + 1) + (size_t)K * (2 * C + 1) + (size_t)kWarps * 32 * ((C + 1) | 1));
-  int occ = 0;
-  switch (CP) {
-    case 8: rc = occupancy_fwd<8>(target_kind, smem, &occ); break;
-    case 16: rc = occupancy_fwd<16>(target_kind, smem, &occ); break;
-    case 24: rc = occupancy_fwd<24>(target_kind, smem, &occ); break;
-    case 32: rc = occupancy_fwd<32>(target_kind, smem, &occ); break;
-    default: rc = occupancy_fwd<64>(target_kind, smem, &occ); break;
-  }
-  if (rc) return rc;
-  ISA_CHECK_ARG(occ >= 1, "disc_loss_fwd: kernel does not fit on an SM (smem %zu)", smem);
-  const int NB = di.num_sms * occ;  // co-resident CTAs
-  int G, grid;
-  if (bs <= NB) { G = NB / bs; grid = G * bs; } else { G = 1; grid = NB; }
-  prm.G = G;
-  prm.strips = (W + 31) / 32;
-  int rowsplits = (G * kWarps) / prm.strips;
-  rowsplits = rowsplits < 1 ? 1 : (rowsplits > H ? H : rowsplits);
-  prm.rpt = (H + rowsplits - 1) / rowsplits;
-  prm.rowsplits = (H + prm.rpt - 1) / prm.rpt;
-  prm.lab_kernel_follows = use_lab ? 1 : 0;
-  switch (CP) {
-    case 8: rc = launch_fwd<8>(prm, grid, smem, stream); break;
-    case 16: rc = launch_fwd<16>(prm, grid, smem, stream); break;
-    case 24: rc = launch_fwd<24>(prm, grid, smem, stream); break;
-    case 32: rc = launch_fwd<32>(prm, grid, smem, stream); break;
-    default: rc = launch_fwd<64>(prm, grid, smem, stream); break;
-  }
-  if (rc || !use_lab) return rc;
-  {
-    const void* fn = nullptr;
-    switch (CP) {
-      case 8: fn = (const void*)disc_fwd_lab_kernel<8>; break;
-      case 16: fn = (const void*)disc_fwd_lab_kernel<16>; break;
-      case 24: fn = (const void*)disc_fwd_lab_kernel<24>; break;
-      case 32: fn = (const void*)disc_fwd_lab_kernel<32>; break;
-      default: fn = (const void*)disc_fwd_lab_kernel<64>; break;
-    }
+  if (pl.route != ROUTE_COL) {
+    LabParams lp;
+    lp.f = prm;
+    lp.f.G = 1; lp.f.strips = 0; lp.f.rowsplits = 0; lp.f.rpt = 0; lp.f.lab_kernel_follows = 0;
+    lp.G = pl.lab_G;
+    lp.chunk = (((H * W + pl.lab_G - 1) / pl.lab_G) + 31) / 32 * 32;
+    lp.priv = pl.priv;
     void* args[] = {(void*)&lp};
-    ISA_CUDA(cudaLaunchCooperativeKernel(fn, dim3(lab_grid), dim3(kThreads), args, lab_smem, stream));
+    ISA_CUDA(cudaLaunchCooperativeKernel(lab_kernel_fn(pl.CP), dim3(pl.lab_grid), dim3(kThreads), args, pl.lab_smem, stream));
   }
   return ISA_OK;
 }
@@ -1310,25 +1358,19 @@ int isa_disc_loss_bwd(const float* emb, const void* target, int target_kind, con
   prm.w_var = w_var; prm.w_dist = w_dist; prm.w_reg = w_reg; prm.w_q = w_q;
   prm.means = means; prm.grad_loss = grad_loss; prm.grad_means = grad_means; prm.grad_emb = grad_emb; prm.q_den = q_den;
 
-  disc_bwd_prep_kernel<<<bs, 128, sizeof(float) * (size_t)K * C, stream>>>(prm);
-  ISA_CUDA(cudaGetLastError());
+  DiscPlan pl;
+  rc = make_plan(target_kind, bs, C, K, H, W, false, di, &pl);
+  if (rc) return rc;
 
-  const int CP = pick_cp(C);
-  const size_t smem = sizeof(float) * 2 * (size_t)K * (CP + 1);
-  const int P = H * W;
-  int gx = (P + kThreads - 1) / kThreads;
-  const int target_ctas = di.num_sms * 8;
-  int per_img = (target_ctas + bs - 1) / bs;
-  if (gx > per_img) gx = per_img;
-  if (gx < 1) gx = 1;
-  dim3 grid(gx, bs);
-  ISA_CHECK_ARG(bs <= 65535, "disc_loss_bwd: bs=%d > 65535", bs);
-  switch (CP) {
-    case 8: return launch_bwd<8>(prm, grid, smem, stream);
-    case 16: return launch_bwd<16>(prm, grid, smem, stream);
-    case 24: return launch_bwd<24>(prm, grid, smem, stream);
-    case 32: return launch_bwd<32>(prm, grid, smem, stream);
-    default: return launch_bwd<64>(prm, grid, smem, stream);
+  disc_bwd_prep_kernel<<<bs, 128, pl.prep_smem, stream>>>(prm);
+  ISA_CUDA(cudaGetLastError());
+  const dim3 grid(pl.bwd_gx, bs);
+  switch (pl.CP) {
+    case 8: return launch_bwd<8>(prm, grid, pl.bwd_smem, stream);
+    case 16: return launch_bwd<16>(prm, grid, pl.bwd_smem, stream);
+    case 24: return launch_bwd<24>(prm, grid, pl.bwd_smem, stream);
+    case 32: return launch_bwd<32>(prm, grid, pl.bwd_smem, stream);
+    default: return launch_bwd<64>(prm, grid, pl.bwd_smem, stream);
   }
 }
 

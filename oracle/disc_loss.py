@@ -44,8 +44,12 @@ def _norm(v, norm, axis):
 
 def discriminative_loss(emb, target, n_objects, max_n_objects, delta_v, delta_d, norm=2,
                         terms=SHIPPED_TERMS, normalize_means=True, dtype=np.float64, want_grad=False,
-                        grad_means=None):
-    """Returns dict(loss, means (bs,K,C), terms (var, dist, reg, qreg)[, grad (bs,C,H,W)])."""
+                        grad_means=None, q_den=None, grad_loss=1.0):
+    """Returns dict(loss, means (bs,K,C), terms (var, dist, reg, qreg)[, grad (bs,C,H,W)]).
+
+    q_den replaces the q-regulariser's denominator int(sum(target)) (the data-parallel run passes
+    global foreground / world size).  grad is the gradient of grad_loss * loss + sum(means * grad_means):
+    grad_loss scales the loss terms' part, not the grad_means part."""
     emb = np.asarray(emb)
     bs, C, H, W = emb.shape
     K = int(max_n_objects)
@@ -83,7 +87,7 @@ def discriminative_loss(emb, target, n_objects, max_n_objects, delta_v, delta_d,
             reg_b[b] = _norm(mu, norm, 1).mean() if n > 0 else np.nan
             cache.append((n, Mb, cnt, mu, r, diff, d, h, Nb))
         fg = M.sum(2)  # bs,P   (all K channels)
-        num = int(fg.sum())
+        num = int(fg.sum()) if q_den is None else q_den
         l2 = np.sqrt(np.sum((X * fg[:, :, None]) ** 2, axis=2))
         qreg = ((l2 - 1) ** 2).sum() / dtype(num) if num != 0 else np.inf
         var_t = var_b.sum() / bs
@@ -104,6 +108,7 @@ def discriminative_loss(emb, target, n_objects, max_n_objects, delta_v, delta_d,
 
     # ---- analytic gradient wrt emb (SURVEY.md Appendix A) ----
     G = np.zeros((bs, P, C), dtype=dtype)
+    gl = dtype(grad_loss)
     with np.errstate(divide="ignore", invalid="ignore"):
         for b in range(bs):
             n, Mb, cnt, mu, r, diff, d, h, Nb = cache[b]
@@ -114,7 +119,7 @@ def discriminative_loss(emb, target, n_objects, max_n_objects, delta_v, delta_d,
             else:
                 dirv = np.sign(diff)
             gs = (2 * h * Mb)[:, :, None] * dirv  # P,n,C : d(m h^2)/dx
-            cdir = w_var / (bs * Nb)
+            cdir = gl * w_var / (bs * Nb)
             G[b] += cdir * gs.sum(1)
             Gam = -cdir * gs.sum(0)  # n,C  dL/dmu_k
             if grad_means is not None:
@@ -122,9 +127,9 @@ def discriminative_loss(emb, target, n_objects, max_n_objects, delta_v, delta_d,
             if w_reg != 0:
                 if norm == 2:
                     nr = np.sqrt(np.sum(mu * mu, 1))
-                    Gam = Gam + (w_reg / bs / n) * np.where(nr[:, None] > 0, mu / np.where(nr > 0, nr, 1)[:, None], 0)
+                    Gam = Gam + (gl * w_reg / bs / n) * np.where(nr[:, None] > 0, mu / np.where(nr > 0, nr, 1)[:, None], 0)
                 else:
-                    Gam = Gam + (w_reg / bs / n) * np.sign(mu)
+                    Gam = Gam + (gl * w_reg / bs / n) * np.sign(mu)
             if w_dist != 0 and n > 1:
                 dm = mu[:, None, :] - mu[None, :, :]
                 e = _norm(dm, norm, 2)
@@ -133,13 +138,13 @@ def discriminative_loss(emb, target, n_objects, max_n_objects, delta_v, delta_d,
                     dire = np.where(e[:, :, None] > 0, dm / np.where(e > 0, e, 1)[:, :, None], 0)
                 else:
                     dire = np.sign(dm)
-                Gam = Gam + (w_dist / bs / (n * (n - 1))) * (-4 * mg[:, :, None] * dire).sum(1)
+                Gam = Gam + (gl * w_dist / bs / (n * (n - 1))) * (-4 * mg[:, :, None] * dire).sum(1)
             if normalize_means:
                 Gam = (Gam - mu * np.sum(mu * Gam, axis=1, keepdims=True)) / r[:, None]
             T = Gam / cnt[:, None]
             G[b] += Mb @ T
         if w_q != 0:
-            cq = w_q / dtype(num)
+            cq = gl * w_q / dtype(num)
             sc = np.where(l2 > 0, 2 * (l2 - 1) * fg * fg / np.where(l2 > 0, l2, 1), 0)
             G += cq * sc[:, :, None] * X
     out["grad"] = np.ascontiguousarray(G.transpose(0, 2, 1)).reshape(bs, C, H, W)
