@@ -37,7 +37,9 @@ def write_prediction(out_dir, image_name, image, fg_seg_pred, ins_seg_pred, n_ob
     np.save(os.path.join(out_dir, image_name + '-n_objects.npy'), n_objects_pred)
 
 
-def build_model_and_prediction(dataset, model_path, seed=0):
+def build_model_and_prediction(dataset, model_path, seed=0, count_head=False):
+    """count_head: build the network with the instance-count head (the checkpoint must have been trained with it) and
+    cluster each image with its predicted count."""
     from isa_b200.model import Model
     from isa_b200.prediction import Prediction
     from isa_b200 import settings
@@ -45,7 +47,7 @@ def build_model_and_prediction(dataset, model_path, seed=0):
     model = Model(dataset, ms.MODEL_NAME, ms.N_CLASSES, ms.MAX_N_OBJECTS,
                   use_instance_segmentation=ms.USE_INSTANCE_SEGMENTATION, use_coords=ms.USE_COORDINATES,
                   load_model_path=model_path or '', usegpu=True, n_embedding=ms.D_MODEL,
-                  n_objects_prediction=ms.N_OBJECTS_PREDICTION,
+                  n_objects_prediction=ms.N_OBJECTS_PREDICTION, count_head=count_head or ms.COUNT_HEAD,
                   net_kwargs=dict(n_units=ms.N_RENET_UNITS, n_head=ms.N_HEAD, d_k=ms.D_K, d_v=ms.D_V))
     prediction = Prediction(ms.IMAGE_HEIGHT, ms.IMAGE_WIDTH, ms.MEAN, ms.STD, False, model, 1, seed=seed, strict=False)
     return model, prediction

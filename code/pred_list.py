@@ -18,6 +18,8 @@ parser.add_argument('--usegpu', action='store_true', default=True)
 parser.add_argument('--output', required=True, help='Path of the output directory')
 parser.add_argument('--dataset', type=str, default='CVPPP')
 parser.add_argument('--seed', type=int, default=0)
+parser.add_argument('--count_head', action='store_true', help='Network with the instance-count head: each image is clustered '
+                    'with its own predicted number of instances (the model must have been trained with --count_head)')
 
 if __name__ == '__main__':
     opt = parser.parse_args()
@@ -25,7 +27,7 @@ if __name__ == '__main__':
     if images_list.ndim > 1:
         images_list = images_list[:, 0]
     image_names = [os.path.splitext(os.path.basename(p))[0] for p in images_list]
-    model, prediction = _common.build_model_and_prediction(opt.dataset, opt.model, opt.seed)
+    model, prediction = _common.build_model_and_prediction(opt.dataset, opt.model, opt.seed, opt.count_head)
     from PIL import Image
     raws = (np.array(Image.open(str(p)).convert('RGB')) for p in images_list)
     kept = []

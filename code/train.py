@@ -30,6 +30,7 @@ parser.add_argument('--synthetic', type=int, default=8, help='Number of syntheti
 parser.add_argument('--target_format', default='compact', choices=['compact', 'reference'],
                     help='compact: uint8 class / label maps (15 MB per 16-image batch); reference: the int64 one-hot tensors of '
                          'lib/dataset.py:354-376 (298 MB), distilled on the device')
+parser.add_argument('--count_head', action='store_true', help='Train the instance-count head as well (count loss added to the cost)')
 parser.add_argument('--cuda_graph', action='store_true', help='Replay forward+backward of the training step from a CUDA graph (fixed batch shape)')
 
 
@@ -67,7 +68,7 @@ if __name__ == '__main__':
     model = Model(opt.dataset, ts.MODEL_NAME, ts.N_CLASSES, ts.MAX_N_OBJECTS,
                   use_instance_segmentation=ts.USE_INSTANCE_SEGMENTATION, use_coords=ts.USE_COORDINATES,
                   load_model_path=opt.model, usegpu=True, n_embedding=ts.D_MODEL, distributed=world > 1,
-                  device=torch.device('cuda', local_rank))
+                  device=torch.device('cuda', local_rank), count_head=opt.count_head or ts.COUNT_HEAD)
     if opt.cuda_graph:
         model.enable_cuda_graph()
     train_loader = SyntheticLoader(opt.synthetic, opt.batchsize, ts, 1000 * rank, opt.target_format)

@@ -344,6 +344,31 @@ int isa_maxpool2x2_fwd(const float* x, int N, int H, int W, int C, float* y, uns
 int isa_maxpool2x2_bwd(const float* gy, const unsigned char* idx, int N, int H, int W, int C, const float* skip_grad,
                        long long skip_pixel_stride, float* gx, isa_stream_t stream);
 
+/* ------------------------------------------------------------------ instance-count tail (ReSeg(count_head=True))
+ * The end of the count branch: conv4's bias + ReLU epilogue, global average pool, the 64 -> 1 linear layer, sigmoid,
+ * count-regression loss and rounding, as one forward and one streaming backward.  The branch is this project's own
+ * specification (archs.py); its float64 restatement is oracle/count_head_ref.py.
+ *   x          [bs][P][C] f32 NHWC: the bias-free conv4 output, finished IN PLACE to y = relu(x + conv_bias) (kept for
+ *              the backward); conv_bias [C], w [C] (the linear layer's weight row), b [1]
+ *   pooled     [bs][C] = mean_p y;  s [bs] = sigmoid(pooled . w + b);  n_pred [bs] i32 = clamp(rint(s * K), 1, K)
+ *              (round half to even, like torch.round)
+ *   n_objects  [bs] i32, or NULL (inference: then loss must be NULL too)
+ *   loss       [1] = mean_b (s_b - n_objects_b / K)^2, or NULL
+ * Backward, with dz_b = grad_loss * 2 (s_b - n_objects_b / K) / bs * s_b (1 - s_b):
+ *   gx [bs][P][C] = (y > 0) dz_b w_c / P;  dconv_bias [C] = sum_{b,p} gx;  dw [C] = sum_b dz_b pooled[b];  db [1] = sum_b dz_b.
+ * workspace  isa_count_head_workspace_bytes(bs, P, C) bytes; hand the SAME buffer, untouched, to the backward (it
+ *            carries the forward's per-(b, c) counts of y > 0, so the bias gradient needs no pass over the map).
+ * Limits: 1 <= bs <= 65535, 1 <= P, C % 4 == 0 and 4 <= C <= 256, 1 <= K <= 254; x, conv_bias, y, gx, w 16-byte
+ * aligned.  A rejected call enqueues nothing.  Deterministic: fixed-order sums, no float atomics. */
+size_t isa_count_head_workspace_bytes(int bs, long long P, int C);
+int isa_count_head_fwd(float* x, const float* conv_bias, const float* w, const float* b, const int* n_objects,
+                       int bs, long long P, int C, int K, float* pooled, float* s, int* n_pred, float* loss,
+                       void* workspace, size_t workspace_bytes, isa_stream_t stream);
+int isa_count_head_bwd(const float* y, const float* pooled, const float* s, const float* w, const int* n_objects,
+                       const float* grad_loss, int bs, long long P, int C, int K,
+                       float* gx, float* dconv_bias, float* dw, float* db,
+                       void* workspace, size_t workspace_bytes, isa_stream_t stream);
+
 /* ------------------------------------------------------------------ fused gradient clipping + Adadelta
  * The tail of the reference's training step (/root/reference/code/lib/model.py:271-281: clip_grad_norm_ then
  * optimizer.step(); settings/CVPPP/training_settings.py: OPTIMIZER 'Adadelta', LEARNING_RATE 1, WEIGHT_DECAY 1e-3,

@@ -12,11 +12,17 @@ and heads are stock cuDNN layers (out of scope, SURVEY.md section 2).
 `forward(training, images, ...)` keeps the reference's calling convention (reseg.py:106) and
 returns `(sem_seg_logits, ins_seg_embedding)`, which is what `Model.predict` unpacks
 (lib/model.py:480-481).
+
+`ReSeg(..., count_head=True)` adds the instance-count branch that reseg.py:13-40 documents as the third head and the
+reference tree never builds; the layer list in `CountBranch` is this project's specification (its float64
+restatement, the oracle of the tests, is oracle/count_head_ref.py).  `forward` then returns a third element,
+`CountFeatures`, whose `evaluate(n_objects)` runs the fused tail (count_head.py).
 """
 import torch
 import torch.nn as nn
 
 from .attention import MultiHeadAttention
+from .count_head import count_tail
 from .pointwise import ConvBiasAct, ConvTransposeBiasAct, MaxPool2x2, pixel_heads, thin_linear
 from .renet import ReNet
 
@@ -78,15 +84,59 @@ class EmbeddingPath(nn.Module):
         return out
 
 
+class CountBranch(nn.Module):
+    """`ins_cls_cnn`, the convolutions of the instance-count branch over the EmbeddingPath output y (N, C, H/4, W/4):
+
+        pool1 MaxPool2x2 -> conv1 3x3 C->64 +ReLU -> conv2 3x3 64->64 +ReLU -> pool2 MaxPool2x2
+        -> conv3 3x3 64->64 +ReLU -> conv4 3x3 64->64 (bias + ReLU in the fused tail, count_head.py)
+
+    `forward` takes pool1's output (ReSeg pools y with the skip to upsampling1, so that both gradients of y are summed in
+    the pooling backward kernel) and returns conv3's output; conv4 is only a parameter holder for the tail."""
+
+    def __init__(self, n_input, n_filters=64):
+        super(CountBranch, self).__init__()
+        self.pool1 = MaxPool2x2()
+        self.conv1 = ConvBiasAct(n_input, n_filters, 3, padding=1, relu=True)
+        self.conv2 = ConvBiasAct(n_filters, n_filters, 3, padding=1, relu=True)
+        self.pool2 = MaxPool2x2()
+        self.conv3 = ConvBiasAct(n_filters, n_filters, 3, padding=1, relu=True)
+        self.conv4 = nn.Conv2d(n_filters, n_filters, 3, padding=1)
+
+    def forward(self, x):
+        return self.conv3(self.pool2(self.conv2(self.conv1(x))))
+
+
+class CountRegressor(nn.Module):
+    """`ins_cls_out`: global average pool -> linear n_filters -> 1 -> sigmoid (all inside the fused tail)."""
+
+    def __init__(self, n_filters=64):
+        super(CountRegressor, self).__init__()
+        self.linear = nn.Linear(n_filters, 1)
+
+
+class CountFeatures(object):
+    """conv3's output of the count branch and the layers of its tail.  evaluate(n_objects=None) -> count_head.CountOutput
+    (loss, s, n_pred, pooled, y): s in (0, 1) is the predicted count / K, n_pred = clamp(round(s K), 1, K) int32;
+    with integer targets n_objects (N,) the loss mean_b (s_b - n_objects_b / K)^2 is computed and differentiable."""
+
+    def __init__(self, x, conv4, linear, max_n_objects):
+        self.x, self.conv4, self.linear, self.max_n_objects = x, conv4, linear, max_n_objects
+
+    def evaluate(self, n_objects=None):
+        return count_tail(self.x, self.conv4, self.linear, self.max_n_objects, n_objects)
+
+
 class ReSeg(nn.Module):
     """See module docstring.  Argument names follow reseg.py:52-55."""
 
     def __init__(self, n_classes, use_instance_seg=True, pretrained=False, use_coordinates=False,
                  use_wae=False, usegpu=True, training=True, n_input=3, n_embedding=24,
-                 n_units=100, n_head=2, d_k=12, d_v=12):
+                 n_units=100, n_head=2, d_k=12, d_v=12, count_head=False, max_n_objects=None):
         super(ReSeg, self).__init__()
         if pretrained:
             raise ValueError("pretrained VGG16 weights cannot be downloaded here; load a state_dict instead")
+        if count_head and not (max_n_objects and 1 <= int(max_n_objects) <= 254):
+            raise ValueError("count_head=True needs max_n_objects in 1..254, got %r" % (max_n_objects,))
         self.n_classes = n_classes
         self.use_instance_seg = use_instance_seg
         self.base = SkipVGG16(n_input)
@@ -100,17 +150,32 @@ class ReSeg(nn.Module):
         self.sem_seg_output = ConvBiasAct(50 + 64, n_classes, kernel_size=(1, 1), stride=(1, 1))
         if use_instance_seg:
             self.ins_seg_output = ConvBiasAct(50 + 64, n_embedding, kernel_size=(1, 1), stride=(1, 1))
+        self.count_head = bool(count_head)
+        if self.count_head:
+            self.max_n_objects = int(max_n_objects)
+            self.ins_cls_cnn = CountBranch(c)
+            self.ins_cls_out = CountRegressor()
 
     def forward(self, training, *_input):
+        """-> (sem_seg_logits, ins_seg_embedding), plus CountFeatures with the count head."""
         x = _input[0]
+        if self.count_head and (x.shape[2] < 16 or x.shape[3] < 16):
+            raise ValueError("the count head pools the 1/4-resolution map twice: input height and width must be >= 16, "
+                             "got %dx%d" % (x.shape[2], x.shape[3]))
         feats, s1, s2 = self.base(x)
         y = self.path(feats)
+        count = None
+        if self.count_head:
+            p, y = self.ins_cls_cnn.pool1.with_skip(y)
+            count = CountFeatures(self.ins_cls_cnn(p), self.ins_cls_cnn.conv4, self.ins_cls_out.linear, self.max_n_objects)
         y = self.relu1(self.upsampling1(y))
         y = torch.cat((y, s2), dim=1)
         y = self.relu2(self.upsampling2(y))
         # both 1x1 heads in one pass over (y | s1) -- the concatenation is never materialised -- straight to the NCHW
         # planes the loss / clustering kernels read
         if self.use_instance_seg:
-            return pixel_heads(y, s1, self.sem_seg_output, self.ins_seg_output)
-        sem_seg_out, _ = pixel_heads(y, s1, self.sem_seg_output)
-        return sem_seg_out, sem_seg_out.argmax(1, keepdim=True).float()
+            out = pixel_heads(y, s1, self.sem_seg_output, self.ins_seg_output)
+        else:
+            sem_seg_out, _ = pixel_heads(y, s1, self.sem_seg_output)
+            out = sem_seg_out, sem_seg_out.argmax(1, keepdim=True).float()
+        return out if count is None else (out[0], out[1], count)

@@ -6,6 +6,7 @@
          lr_drop_factor, lr_drop_patience, optimize_bg, optimizer, train_cnn, n_epochs, class_weights,
          train_loader, test_loader, model_save_path, debug)
     .predict(images) -> (sem_probs (b,n_classes,h,w), embeddings (b,C,h,w), n_objects IntTensor (b,1))
+    (n_objects: the trained count head's prediction with count_head=True, else the constant n_objects_prediction)
 
 The reference file cannot be parsed by Python >= 3.7 (`cuda(async=True)`, model.py:221-225,476) and its
 training step takes `ins_cost` from a NaN-producing decoder (SURVEY.md R3/R5); this is a rewrite with
@@ -13,8 +14,9 @@ the same surface where the step is the designed one (SURVEY.md section 3.1):
     sem_logits, emb = net(True, images); ins_cost, means = criterion_discriminative(emb, ins, n, K)
     cost = ins_cost + CE + Dice; backward; clip_grad_norm_; optimizer.step()
 Extras: `train_step(...)` (the public face of the reference's private __minibatch), device-resident
-`predict_device(...)`, and single-node data parallelism (`distributed=True`): one process per GPU,
-parameters replicated, ONE flat-bucket NCCL all-reduce of the gradients per step.
+`predict_device(...)` / `predict_device_with_counts(...)`, the optional instance-count head (`count_head=True`), and
+single-node data parallelism (`distributed=True`): one process per GPU, parameters replicated, ONE flat-bucket NCCL
+all-reduce of the gradients per step.
 visdom plotting and the pickle dumps to a hard-coded path (model.py:55,454-457) are dropped.
 """
 import os
@@ -37,7 +39,8 @@ class Model(object):
     def __init__(self, dataset, model_name, n_classes, max_n_objects, wae_opt=None,
                  use_instance_segmentation=False, use_wae=False, use_coords=False,
                  load_model_path='', load_decoder_model_path='', usegpu=True,
-                 n_input=3, n_embedding=24, n_objects_prediction=16, distributed=False, device=None, net_kwargs=None):
+                 n_input=3, n_embedding=24, n_objects_prediction=16, distributed=False, device=None, net_kwargs=None,
+                 count_head=False):
         self.dataset = dataset
         self.model_name = model_name
         self.n_classes = n_classes
@@ -49,6 +52,7 @@ class Model(object):
         self.use_wae = use_wae
         self.usegpu = usegpu
         self.n_objects_prediction = int(n_objects_prediction)
+        self.count_head = bool(count_head)
         assert self.dataset in ['CVPPP', 'Cityscapes']
         assert self.model_name in ['ReSeg']
         if not usegpu:
@@ -57,7 +61,8 @@ class Model(object):
         self.device = torch.device(device) if device is not None else torch.device('cuda', torch.cuda.current_device())
         self.model = ReSeg(self.n_classes, self.use_instance_segmentation, pretrained=False,
                            use_coordinates=self.use_coords, use_wae=use_wae, usegpu=True,
-                           n_input=n_input, n_embedding=n_embedding, **(net_kwargs or {}))
+                           n_input=n_input, n_embedding=n_embedding, count_head=self.count_head,
+                           max_n_objects=self.max_n_objects, **(net_kwargs or {}))
         self.__load_weights()
         torch.backends.cudnn.benchmark = True          # model.py:50-52
         self.model.to(self.device).to(memory_format=torch.channels_last)
@@ -222,12 +227,16 @@ class Model(object):
 
     def __fwd_bwd(self, images, sem_map, ins, nobj, criterion_type, training, q_den):
         """Forward, losses and (training) zero_grad + backward on COMPACT device targets; returns the metrics dict of
-        model.py:242-269."""
+        model.py:242-269.  With the count head, cost += 'Count Cost' = mean_b (s_b - n_objects_b / K)^2 (weight 1) and
+        'Count |DiC|' = mean_b |n_pred_b - n_objects_b| is reported; both stay device scalars (nothing synchronises, the
+        step still captures in a CUDA graph).  Data parallel: the shards are equal-sized and the gradients are averaged,
+        so the per-rank batch mean of the count loss gives the global-batch gradient with no collective of its own."""
         self.model.train(training)
         images = images.contiguous(memory_format=torch.channels_last)
         out_metrics = dict()
         with torch.set_grad_enabled(training):
-            sem_seg_predictions, ins_seg_predictions = self.model(training, images)
+            outputs = self.model(training, images)
+            sem_seg_predictions, ins_seg_predictions = outputs[0], outputs[1]
             cost = 0
             if self.use_instance_segmentation:
                 ins_cost, _means = self.criterion_discriminative(ins_seg_predictions, ins, nobj, self.max_n_objects,
@@ -242,6 +251,11 @@ class Model(object):
                 if criterion_type in ['Dice', 'Multi']:
                     cost = cost + dice_cost
                     out_metrics['Dice Cost'] = dice_cost.detach()
+            if self.count_head:
+                count = outputs[2].evaluate(nobj)
+                cost = cost + count.loss
+                out_metrics['Count Cost'] = count.loss.detach()
+                out_metrics['Count |DiC|'] = (count.n_pred - nobj).abs().float().mean()
             out_metrics['Cost'] = cost.detach()
         if training:
             if hasattr(self.optimizer, 'flat_grad'):
@@ -338,18 +352,27 @@ class Model(object):
 
     # ------------------------------------------------------------------ predict (model.py:466-499)
     @torch.no_grad()
-    def predict_device(self, images):
-        """-> (sem_probs, embeddings) on the device, nothing synchronised."""
+    def predict_device_with_counts(self, images):
+        """-> (sem_probs, embeddings, n_pred) on the device, nothing synchronised; n_pred (b,) int32 is the count head's
+        clamp(round(s K), 1, K), or None without the head."""
         assert len(images.size()) == 4  # b, c, h, w
         self.model.eval()
         images = images.to(self.device, non_blocking=True).contiguous(memory_format=torch.channels_last)
-        sem_seg_predictions, ins_seg_predictions = self.model(False, images)
-        sem_seg_predictions = torch.nn.functional.softmax(sem_seg_predictions, dim=1)
-        return sem_seg_predictions, ins_seg_predictions
+        outputs = self.model(False, images)
+        sem_seg_predictions = torch.nn.functional.softmax(outputs[0], dim=1)
+        n_pred = outputs[2].evaluate().n_pred if self.count_head else None
+        return sem_seg_predictions, outputs[1], n_pred
+
+    def predict_device(self, images):
+        """-> (sem_probs, embeddings) on the device, nothing synchronised."""
+        return self.predict_device_with_counts(images)[:2]
 
     def predict(self, images):
-        sem, ins = self.predict_device(images)
+        sem, ins, n_pred = self.predict_device_with_counts(images)
         if self.use_instance_segmentation:
-            n_objects_predictions = torch.IntTensor([[self.n_objects_prediction]] * images.size(0))
+            if n_pred is not None:
+                n_objects_predictions = n_pred.cpu().reshape(-1, 1)
+            else:
+                n_objects_predictions = torch.IntTensor([[self.n_objects_prediction]] * images.size(0))
             return sem.cpu(), ins.cpu(), n_objects_predictions
         return sem.cpu()

@@ -7,7 +7,9 @@
 The CPU hop of the reference (.cpu().numpy() -> np.stack gather -> sklearn KMeans -> python scatter loop
 -> cv2.resize, prediction.py:57-85,105-108) is replaced by the device pipeline of clustering.py:
 argmax + foreground compaction, k-means++/Lloyd for all 35 restarts in one kernel, label scatter and
-nearest up-sampling; only the two final uint8 masks are copied back.  New argument `seed` (the reference
+nearest up-sampling; only the two final uint8 masks are copied back.  A model with the count head
+(`Model(count_head=True)`) clusters each image with its own predicted count: that count is k, a host argument of the
+k-means kernels, so its 4 bytes are read back before the clustering is enqueued.  New argument `seed` (the reference
 never seeds KMeans, so its output is not reproducible; here the default is 0).
 Input images: RGB -> bilinear resize -> ToTensor -> Normalize(mean, std) (3 channels; the reference's
 21-channel colour-space expansion needs scikit-image, which is not installed, and is data
@@ -77,10 +79,11 @@ class Prediction(object):
 
     # ---- predict (prediction.py:87-124)
     def predict_array(self, raw_image):
-        """raw_image HxWx3 uint8 -> (sem_seg uint8 HxW, ins_seg uint8 HxW, n_objects); one device->host copy."""
+        """raw_image HxWx3 uint8 -> (sem_seg uint8 HxW, ins_seg uint8 HxW, n_objects); one device->host copy of the masks
+        (and, with the count head, one of the 4-byte count before the clustering)."""
         image, image_height, image_width = self.image_to_tensor(raw_image)
-        sem, emb = self.model.predict_device(image.unsqueeze(0).pin_memory())
-        n = self.model.n_objects_prediction
+        sem, emb, n_pred = self.model.predict_device_with_counts(image.unsqueeze(0).pin_memory())
+        n = self.model.n_objects_prediction if n_pred is None else int(n_pred[0])
         _, _, ins_up, cls_up, res = self.cluster_device(sem[0], emb[0], n, image_height, image_width)
         both = torch.stack([cls_up, ins_up]).cpu()     # the only D2H copy (also the sync point)
         if self.strict:
@@ -96,7 +99,9 @@ class Prediction(object):
     def predict_many(self, raw_images, prefetch=2):
         """Pipelined `predict_array` over an iterable of HxWx3 uint8 images (what pred_list.py does with a list of
         paths): a worker thread resizes / normalises / pins image i+1 (PIL releases the GIL) while the device works on
-        image i, and the masks of image i are copied back asynchronously while image i+1 is enqueued.
+        image i, and the masks of image i are copied back asynchronously while image i+1 is enqueued.  The network of
+        image i+1 is enqueued before the clustering of image i, so that waiting for image i's predicted count (count head)
+        never leaves the device idle, except on the first image.
         Yields (sem_seg uint8 HxW, ins_seg uint8 HxW, n_objects) in order; results are identical to predict_array."""
         import queue
         import threading
@@ -116,15 +121,47 @@ class Prediction(object):
                 q.put(None)
 
         threading.Thread(target=producer, daemon=True).start()
-        n = self.model.n_objects_prediction
-        pending = None
         ring = {}          # (h, w) -> two pinned staging buffers used alternately (masks + the k-means info words)
+        counts = [torch.empty(1, dtype=torch.int32).pin_memory() for _ in range(2)]   # predicted counts, alternately
+
+        def finish(p):
+            host, info, ev, n = p
+            ev.synchronize()
+            if int(info[0]) != 0:
+                msg = ("n_samples=%d should be >= n_clusters." % int(info[2]) if int(info[0]) == 1
+                       else "Input X contains NaN or infinity.")
+                if self.strict:
+                    raise ValueError(msg)
+                sys.stderr.write("warning: image not clustered (%s); writing an empty instance mask\n" % msg)
+                return host[0].numpy().copy(), np.zeros_like(host[1].numpy()), 0
+            return host[0].numpy().copy(), host[1].numpy().copy(), n
+
+        staged = None      # network enqueued, clustering not yet: (sem, emb, h, w, pinned count or None, its event)
+        pending = None     # clustering enqueued, masks on their way to the host: (host, host_info, event, n)
+        n_images = 0
         turn = 0
         while True:
             item = q.get()
+            nxt = None
             if item is not None:
                 image, h, w = item
-                sem, emb = self.model.predict_device(image)
+                sem, emb, n_pred = self.model.predict_device_with_counts(image)
+                host_n = ev_n = None
+                if n_pred is not None:
+                    host_n = counts[n_images & 1]
+                    host_n.copy_(n_pred[:1], non_blocking=True)
+                    ev_n = torch.cuda.Event()
+                    ev_n.record(torch.cuda.current_stream(dev))
+                n_images += 1
+                nxt = (sem, emb, h, w, host_n, ev_n)
+            cur = None
+            if staged is not None:
+                sem, emb, h, w, host_n, ev_n = staged
+                if host_n is None:
+                    n = self.model.n_objects_prediction
+                else:
+                    ev_n.synchronize()       # the device is already running the next image's network
+                    n = int(host_n[0])
                 _, _, ins_up, cls_up, res = self.cluster_device(sem[0], emb[0], n, h, w)
                 bufs = ring.get((h, w))
                 if bufs is None:
@@ -137,24 +174,15 @@ class Prediction(object):
                 host_info.copy_(res.info, non_blocking=True)
                 ev = torch.cuda.Event()
                 ev.record(torch.cuda.current_stream(dev))
-                cur = (host, host_info, ev)
-            else:
-                cur = None
+                cur = (host, host_info, ev, n)
+            staged = nxt
             if pending is not None:
-                host_p, info_p, ev_p = pending
-                ev_p.synchronize()
-                if int(info_p[0]) != 0:
-                    msg = ("n_samples=%d should be >= n_clusters." % int(info_p[2]) if int(info_p[0]) == 1
-                           else "Input X contains NaN or infinity.")
-                    if self.strict:
-                        raise ValueError(msg)
-                    sys.stderr.write("warning: image not clustered (%s); writing an empty instance mask\n" % msg)
-                    yield host_p[0].numpy().copy(), np.zeros_like(host_p[1].numpy()), 0
-                else:
-                    yield host_p[0].numpy().copy(), host_p[1].numpy().copy(), n
-            if cur is None:
-                break
+                yield finish(pending)
             pending = cur
+            if item is None:
+                break
+        if pending is not None:
+            yield finish(pending)
         if failure:
             raise failure[0]
 

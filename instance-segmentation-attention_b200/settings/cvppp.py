@@ -35,6 +35,9 @@ class ModelSettings(DataSettings):
         self.D_INNER = 40
         self.N_RENET_UNITS = 100
         self.N_OBJECTS_PREDICTION = 16   # lib/model.py:496 hard-codes 16
+        # trained instance-count head (archs.ReSeg(count_head=True)): each image is clustered with its own predicted count
+        # instead of N_OBJECTS_PREDICTION
+        self.COUNT_HEAD = False
 
 
 class TrainingSettings(ModelSettings):
