@@ -1,8 +1,12 @@
 """train.py -- training entry point with the reference's flags (/root/reference/code/train.py:18-37).
-The reference reads LMDB databases (lmdb is not installed and no dataset ships); `--synthetic N` trains on
-N seeded CVPPP-shaped synthetic batches instead, which is also what bench.py measures.  Launch one process
-per GPU with torchrun for single-node data parallelism:
+The reference reads LMDB databases (lmdb is not installed).  `--train_list L --val_list V --gt_dir D` trains on a
+directory of annotated images instead (the CVPPP layout pred_list.py and evaluate.py read: `<base>_rgb.png` listed in
+L and V, `<base>_label.png` under D), decoded once into device memory and augmented on the device with the flags and
+seed of the settings class (isa_b200.augment).  Without `--train_list`, `--synthetic N` trains on N seeded
+CVPPP-shaped synthetic batches, which is also what bench.py measures.  Launch one process per GPU with torchrun for
+single-node data parallelism:
 
+    python code/train.py --output out_dir --train_list train.lst --val_list val.lst --gt_dir A1 --batchsize 16
     python code/train.py --output out_dir --synthetic 8 --nepochs 2 --batchsize 16
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 code/train.py ...
 """
@@ -26,7 +30,10 @@ parser.add_argument('--debug', action='store_true')
 parser.add_argument('--nworkers', type=int, default=2)
 parser.add_argument('--dataset', type=str, default='CVPPP')
 parser.add_argument('--output', default='models', help='Directory for checkpoints and logs')
-parser.add_argument('--synthetic', type=int, default=8, help='Number of synthetic minibatches per epoch')
+parser.add_argument('--synthetic', type=int, default=8, help='Number of synthetic minibatches per epoch (without --train_list)')
+parser.add_argument('--train_list', default='', help='Text file of training image paths (<base>_rgb.png); trains on them instead of synthetic batches')
+parser.add_argument('--val_list', default='', help='Text file of validation image paths (with --train_list)')
+parser.add_argument('--gt_dir', default='', help='Directory with <base>_label.png for every listed image (with --train_list)')
 parser.add_argument('--target_format', default='compact', choices=['compact', 'reference'],
                     help='compact: uint8 class / label maps (15 MB per 16-image batch); reference: the int64 one-hot tensors of '
                          'lib/dataset.py:354-376 (298 MB), distilled on the device')
@@ -71,8 +78,20 @@ if __name__ == '__main__':
                   device=torch.device('cuda', local_rank), count_head=opt.count_head or ts.COUNT_HEAD)
     if opt.cuda_graph:
         model.enable_cuda_graph()
-    train_loader = SyntheticLoader(opt.synthetic, opt.batchsize, ts, 1000 * rank, opt.target_format)
-    test_loader = SyntheticLoader(max(1, opt.synthetic // 4), opt.batchsize, ts, 500000 + 1000 * rank, opt.target_format)
+    if opt.train_list:
+        if not (opt.val_list and opt.gt_dir):
+            parser.error('--train_list needs --val_list and --gt_dir')
+        from isa_b200 import augment
+        flags = augment.flags_from_settings(ts)
+        dev = torch.device('cuda', local_rank)
+        stores = [augment.load_store(p, opt.gt_dir, ts.MAX_N_OBJECTS, ts.IMAGE_HEIGHT, ts.IMAGE_WIDTH, ts.MEAN, ts.STD, dev)
+                  for p in (opt.train_list, opt.val_list)]
+        train_loader, test_loader = [augment.AugmentLoader(st, opt.batchsize * world, ts.IMAGE_HEIGHT, ts.IMAGE_WIDTH, flags,
+                                                           ts.SEED, train, rank, world)
+                                     for st, train in zip(stores, (True, False))]
+    else:
+        train_loader = SyntheticLoader(opt.synthetic, opt.batchsize, ts, 1000 * rank, opt.target_format)
+        test_loader = SyntheticLoader(max(1, opt.synthetic // 4), opt.batchsize, ts, 500000 + 1000 * rank, opt.target_format)
     model.fit(ts.CRITERION, ts.DELTA_VAR, ts.DELTA_DIST, ts.NORM, ts.LEARNING_RATE, ts.WEIGHT_DECAY, ts.CLIP_GRAD_NORM,
               ts.LR_DROP_FACTOR, ts.LR_DROP_PATIENCE, ts.OPTIMIZE_BG, ts.OPTIMIZER, ts.TRAIN_CNN, opt.nepochs,
               ts.CLASS_WEIGHTS, train_loader, test_loader, os.path.join(opt.output, opt.dataset), opt.debug)

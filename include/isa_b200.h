@@ -369,6 +369,35 @@ int isa_count_head_bwd(const float* y, const float* pooled, const float* s, cons
                        float* gx, float* dconv_bias, float* dw, float* db,
                        void* workspace, size_t workspace_bytes, isa_stream_t stream);
 
+/* ------------------------------------------------------------------ training-set augmentation (isa_b200.augment)
+ * Gathers a batch of augmented training samples from a device-resident store of decoded images.  The geometry (which
+ * maps are drawn) is the host's; this call applies them.  Its numpy restatement is oracle/augment_ref.py.
+ *   rgb        [sum h*w][3] u8 and labels [sum h*w] u8 (ids 0..n-1, 255 = background): the images, packed
+ *   store      [n_images][3] i64 = (pixel offset, h, w) of each image; 1 <= h, w <= 32767, offset + h*w <= store_pixels
+ *   params     [b][7] i64 = (source image index, a0..a5): the inverse map output -> source in Q32.32 fixed point,
+ *              |a_i| < 2^44.  Output pixel (x, y) reads the source at, exactly in int64 and in units of 2^-33,
+ *                u = a0 (2x+1) + a1 (2y+1) + 2 a2,   v = a3 (2x+1) + a4 (2y+1) + 2 a5
+ *              label = nearest pixel (u >> 33, v >> 33), 255 outside the source; rgb = bilinear from the four taps
+ *              around (u - 2^32, v - 2^32), taps outside the source read 0, fp32 weights from the low 33 bits.
+ *   h_mean_std [6] f32 on the HOST: mean[3], std[3];  image = (rgb / 255 - mean) / std
+ * Outputs, in the layouts Model.train_step reads:
+ *   image [b][H][W][3] f32 (a (b,3,H,W) tensor in channels_last), sem [b][H][W] u8 = (ins != 255),
+ *   ins [b][H][W] u8, n_objects [b] i32.
+ * The ids present in a sample are renumbered 0..n-1 in ascending order of the source id (nearest sampling, rotation
+ * and cutting drop instances); n_objects = n.  A sample left with no instance is rendered again through the plain
+ * resize map (a0 = round(w 2^32 / W), a4 = round(h 2^32 / H), the rest 0), so n_objects is 0 only if that view has
+ * no instance either.  A map that breaks the limit above counts as a view with no instance, so the sample gets the
+ * plain view; a sample whose source index or store entry is invalid is written black and empty (n_objects 0).
+ * Integer atomics only: the same call writes the same bytes.
+ * workspace  isa_augment_workspace_bytes(b) bytes, 4-byte aligned.
+ * Limits: 1 <= b <= 65535, 1 <= H, W <= 32767, std non-zero (else ISA_ERR_BAD_ARG; a rejected call
+ * enqueues nothing). */
+size_t isa_augment_workspace_bytes(int b);
+int isa_augment(const unsigned char* rgb, const unsigned char* labels, const long long* store, int n_images,
+                long long store_pixels, const long long* params, int b, int H, int W, const float* h_mean_std,
+                float* image, unsigned char* sem, unsigned char* ins, int* n_objects,
+                void* workspace, size_t workspace_bytes, isa_stream_t stream);
+
 /* ------------------------------------------------------------------ fused gradient clipping + Adadelta
  * The tail of the reference's training step (/root/reference/code/lib/model.py:271-281: clip_grad_norm_ then
  * optimizer.step(); settings/CVPPP/training_settings.py: OPTIMIZER 'Adadelta', LEARNING_RATE 1, WEIGHT_DECAY 1e-3,

@@ -119,6 +119,10 @@ SIGNATURES = {
                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "isa_count_head_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_longlong, c_int, c_int,
                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    # training-set augmentation
+    "isa_augment_workspace_bytes": (c_size_t, [c_int]),
+    "isa_augment": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_longlong, c_void_p, c_int, c_int, c_int, c_void_p,
+                            c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "isa_adadelta_workspace_bytes": (c_size_t, []),
     "isa_adadelta_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_float, c_float, c_float, c_float, c_float,
                                   c_void_p, c_void_p, c_size_t, c_void_p]),
@@ -157,7 +161,7 @@ KERNELS_PER_CALL = {
     "isa_readout_fwd": 1, "isa_readout_bwd": 1, "isa_local_attention_fwd": 1, "isa_local_attention_bwd": 2,
     "isa_bias_act_fwd": 1, "isa_bias_act_bwd": 2, "isa_add_layernorm_fwd": 1, "isa_add_layernorm_bwd": 2,
     "isa_pixel_heads_fwd": 1, "isa_pixel_heads_bwd": 1, "isa_pixel_heads_wgrad": 2,
-    "isa_maxpool2x2_fwd": 1, "isa_maxpool2x2_bwd": 1, "isa_count_head_fwd": 2, "isa_count_head_bwd": 1, "isa_adadelta_step": 2,
+    "isa_maxpool2x2_fwd": 1, "isa_maxpool2x2_bwd": 1, "isa_count_head_fwd": 2, "isa_count_head_bwd": 1, "isa_augment": 3, "isa_adadelta_step": 2,
     "isa_renet_proj_fwd": 2, "isa_renet_proj_dx": 2, "isa_renet_proj_wgrad": 2,
     "isa_seg_losses_fwd": 1, "isa_seg_losses_bwd": 1, "isa_onehot_argmax": 1, "isa_sbd": 2,
 }

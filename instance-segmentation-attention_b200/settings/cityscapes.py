@@ -26,3 +26,8 @@ class TrainingSettings(_CVPPPTrainingSettings):
         self.MAX_N_OBJECTS = 64
         self.IMAGE_HEIGHT = 1024
         self.IMAGE_WIDTH = 2048
+        # street scenes have an up: horizontal flips only
+        self.VERTICAL_FLIPPING = False
+        self.TRANSPOSING = False
+        self.ROTATION_90X = False
+        self.ROTATION = False
