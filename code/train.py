@@ -2,9 +2,11 @@
 The reference reads LMDB databases (lmdb is not installed).  `--train_list L --val_list V --gt_dir D` trains on a
 directory of annotated images instead (the CVPPP layout pred_list.py and evaluate.py read: `<base>_rgb.png` listed in
 L and V, `<base>_label.png` under D), decoded once into device memory and augmented on the device with the flags and
-seed of the settings class (isa_b200.augment).  Without `--train_list`, `--synthetic N` trains on N seeded
-CVPPP-shaped synthetic batches, which is also what bench.py measures.  Launch one process per GPU with torchrun for
-single-node data parallelism:
+seed of the settings class (isa_b200.augment).  `--score_every N` also scores the V images every N epochs by the SBD,
+|DiC| and foreground dice that pred_list.py + evaluate.py --empty_as_zero report (validation_scores.log, on the device:
+isa_b200.scoring), and `--select_by sbd` keeps the checkpoints of the best mean SBD instead of the best validation
+cost.  Without `--train_list`, `--synthetic N` trains on N seeded CVPPP-shaped synthetic batches, which is also what
+bench.py measures.  Launch one process per GPU with torchrun for single-node data parallelism:
 
     python code/train.py --output out_dir --train_list train.lst --val_list val.lst --gt_dir A1 --batchsize 16
     python code/train.py --output out_dir --synthetic 8 --nepochs 2 --batchsize 16
@@ -39,6 +41,10 @@ parser.add_argument('--target_format', default='compact', choices=['compact', 'r
                          'lib/dataset.py:354-376 (298 MB), distilled on the device')
 parser.add_argument('--count_head', action='store_true', help='Train the instance-count head as well (count loss added to the cost)')
 parser.add_argument('--cuda_graph', action='store_true', help='Replay forward+backward of the training step from a CUDA graph (fixed batch shape)')
+parser.add_argument('--score_every', type=int, default=0, help='Score the --val_list images by SBD, |DiC| and FG dice every N epochs '
+                    'and after the last one, as pred_list.py + evaluate.py --empty_as_zero would (0 = off) [Default: 0]')
+parser.add_argument('--select_by', default='cost', choices=['cost', 'sbd'], help='Keep the checkpoints of the best validation '
+                    'cost, or of the best mean SBD of the scored epochs (needs --score_every) [Default: cost]')
 
 
 class SyntheticLoader(object):
@@ -68,6 +74,12 @@ class SyntheticLoader(object):
 if __name__ == '__main__':
     opt = parser.parse_args()
     assert opt.dataset in ['CVPPP', 'Cityscapes']
+    if opt.score_every < 0:
+        parser.error('--score_every must be >= 0')
+    if opt.score_every and not opt.train_list:
+        parser.error('--score_every needs --train_list, --val_list and --gt_dir: the synthetic batches have no label files')
+    if opt.select_by == 'sbd' and not opt.score_every:
+        parser.error('--select_by sbd needs --score_every')
     ts = settings.CVPPPTrainingSettings() if opt.dataset == 'CVPPP' else settings.CityscapesTrainingSettings()
     rank, world, local_rank = parallel.init_from_env()
     torch.cuda.set_device(local_rank)
@@ -75,9 +87,11 @@ if __name__ == '__main__':
     model = Model(opt.dataset, ts.MODEL_NAME, ts.N_CLASSES, ts.MAX_N_OBJECTS,
                   use_instance_segmentation=ts.USE_INSTANCE_SEGMENTATION, use_coords=ts.USE_COORDINATES,
                   load_model_path=opt.model, usegpu=True, n_embedding=ts.D_MODEL, distributed=world > 1,
+                  n_objects_prediction=ts.N_OBJECTS_PREDICTION,
                   device=torch.device('cuda', local_rank), count_head=opt.count_head or ts.COUNT_HEAD)
     if opt.cuda_graph:
         model.enable_cuda_graph()
+    scorer = None
     if opt.train_list:
         if not (opt.val_list and opt.gt_dir):
             parser.error('--train_list needs --val_list and --gt_dir')
@@ -89,9 +103,16 @@ if __name__ == '__main__':
         train_loader, test_loader = [augment.AugmentLoader(st, opt.batchsize * world, ts.IMAGE_HEIGHT, ts.IMAGE_WIDTH, flags,
                                                            ts.SEED, train, rank, world)
                                      for st, train in zip(stores, (True, False))]
+        if opt.score_every:
+            from isa_b200.scoring import InstanceScorer
+            # the k-means settings of pred_list.py (seed 0, 35 restarts, 500 iterations): the logged scores are the
+            # ones pred_list.py + evaluate.py --empty_as_zero give for the same checkpoint
+            scorer = InstanceScorer(opt.val_list, opt.gt_dir, ts.IMAGE_HEIGHT, ts.IMAGE_WIDTH, ts.MEAN, ts.STD,
+                                    ts.MAX_N_OBJECTS, dev, seed=0, n_init=35, max_iter=500, rank=rank, world=world)
     else:
         train_loader = SyntheticLoader(opt.synthetic, opt.batchsize, ts, 1000 * rank, opt.target_format)
         test_loader = SyntheticLoader(max(1, opt.synthetic // 4), opt.batchsize, ts, 500000 + 1000 * rank, opt.target_format)
     model.fit(ts.CRITERION, ts.DELTA_VAR, ts.DELTA_DIST, ts.NORM, ts.LEARNING_RATE, ts.WEIGHT_DECAY, ts.CLIP_GRAD_NORM,
               ts.LR_DROP_FACTOR, ts.LR_DROP_PATIENCE, ts.OPTIMIZE_BG, ts.OPTIMIZER, ts.TRAIN_CNN, opt.nepochs,
-              ts.CLASS_WEIGHTS, train_loader, test_loader, os.path.join(opt.output, opt.dataset), opt.debug)
+              ts.CLASS_WEIGHTS, train_loader, test_loader, os.path.join(opt.output, opt.dataset), opt.debug,
+              scorer=scorer, score_every=max(opt.score_every, 1), select_by=opt.select_by)

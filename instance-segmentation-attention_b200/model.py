@@ -4,7 +4,7 @@
           use_wae=True, use_coords=False, load_model_path='', load_decoder_model_path='', usegpu=True)
     .fit(criterion_type, delta_var, delta_dist, norm, learning_rate, weight_decay, clip_grad_norm,
          lr_drop_factor, lr_drop_patience, optimize_bg, optimizer, train_cnn, n_epochs, class_weights,
-         train_loader, test_loader, model_save_path, debug)
+         train_loader, test_loader, model_save_path, debug, scorer=None, score_every=1, select_by='cost')
     .predict(images) -> (sem_probs (b,n_classes,h,w), embeddings (b,C,h,w), n_objects IntTensor (b,1))
     (n_objects: the trained count head's prediction with count_head=True, else the constant n_objects_prediction)
 
@@ -28,7 +28,7 @@ import torch.distributed as dist
 import torch.optim as optim
 from torch.optim.lr_scheduler import ReduceLROnPlateau
 
-from . import _lib, parallel
+from . import _lib, parallel, scoring
 from .archs import ReSeg
 from .losses import DiscriminativeLoss, label_fg_count, onehot_to_labels
 from .seg_losses import DiceLoss, SegLosses, class_map
@@ -296,8 +296,19 @@ class Model(object):
     # ------------------------------------------------------------------ fit (model.py:358-464)
     def fit(self, criterion_type, delta_var, delta_dist, norm, learning_rate, weight_decay, clip_grad_norm,
             lr_drop_factor, lr_drop_patience, optimize_bg, optimizer, train_cnn, n_epochs, class_weights,
-            train_loader, test_loader, model_save_path, debug=False):
+            train_loader, test_loader, model_save_path, debug=False, scorer=None, score_every=1, select_by='cost'):
+        """scorer (scoring.InstanceScorer): score the validation images by SBD, |DiC| and FG dice after the validation
+        pass of every score_every-th epoch and of the last one, into model.score_history as (epoch, SBD, |DiC|,
+        FgDice, unclustered); rank 0 also appends them to validation_scores.log.  select_by='sbd' keeps a checkpoint on each scored epoch whose mean SBD is >= the best so
+        far, instead of each epoch whose validation cost is <= the best so far ('cost').  ReduceLROnPlateau steps on
+        the validation cost either way."""
         assert criterion_type in ['CE', 'Dice', 'Multi']
+        if select_by not in ('cost', 'sbd'):
+            raise ValueError("select_by=%r: expected 'cost' or 'sbd'" % (select_by,))
+        if select_by == 'sbd' and scorer is None:
+            raise ValueError("select_by='sbd' needs a scorer")
+        if int(score_every) < 1:
+            raise ValueError("score_every=%r: must be >= 1" % (score_every,))
         rank0 = (not self.distributed) or dist.get_rank() == 0
         if rank0:
             os.makedirs(model_save_path, exist_ok=True)
@@ -305,27 +316,46 @@ class Model(object):
             validation_log_file = open(os.path.join(model_save_path, 'validation.log'), 'w')
             training_log_file.write('Epoch,Cost\n')
             validation_log_file.write('Epoch,Cost\n')
+            if scorer is not None:
+                scores_log_file = open(os.path.join(model_save_path, 'validation_scores.log'), 'w')
+                scores_log_file.write('Epoch,' + ','.join(scoring.COLUMNS) + '\n')
         self.define_criterion(class_weights, delta_var, delta_dist, norm=norm, optimize_bg=optimize_bg, criterion=criterion_type)
         if not train_cnn:
             for p in self.model.base.parameters():
                 p.requires_grad = False
         self.define_optimizer(learning_rate, weight_decay, lr_drop_factor, lr_drop_patience, optimizer=optimizer)
         best_val_cost = np.inf
+        best_sbd = scoring.BestSBD()
         history = []
+        self.score_history = []
         for epoch in range(n_epochs):
             t0 = time.time()
             train_metrics = self.__run_epoch(train_loader, clip_grad_norm, 'training')
             val_metrics = self.__run_epoch(test_loader, 0.0, 'test')
             train_cost, val_cost = train_metrics['Cost'], val_metrics['Cost']
+            t_epoch = time.time() - t0
+            scores = None
+            if scorer is not None and scoring.is_scored_epoch(epoch, n_epochs, int(score_every)):
+                t1 = time.time()
+                scores = scoring.epoch_scores(scorer.score(self), scorer.n_images, self.device)
+                self.score_history.append((epoch,) + scores)
             self.lr_scheduler.step(val_cost)
             history.append((epoch, train_cost, val_cost))
             if rank0:
                 print('Epoch : [{}/{}] - [{:.1f}s]  Training Cost {:.5f} | Validation Cost {:.5f}'.format(
-                    epoch, n_epochs, time.time() - t0, train_cost, val_cost))
-                if val_cost <= best_val_cost:
+                    epoch, n_epochs, t_epoch, train_cost, val_cost))
+                if scores is not None:
+                    print('Epoch : [{}/{}] - [{:.1f}s]  Validation SBD {:.5f} | |DiC| {:.4f} | FG Dice {:.5f} | '
+                          'unclustered {}/{}'.format(epoch, n_epochs, time.time() - t1, scores[0], scores[1], scores[2],
+                                                     scores[3], scorer.n_images))
+                    scores_log_file.write('{},{},{},{},{}\n'.format(epoch, *scores))
+                    scores_log_file.flush()
+                lr = self.optimizer.param_groups[0]['lr']
+                if select_by == 'cost' and val_cost <= best_val_cost:
                     best_val_cost = val_cost
-                    lr = self.optimizer.param_groups[0]['lr']
                     torch.save(self.model.state_dict(), os.path.join(model_save_path, 'model_{}_{}_{}.pth'.format(epoch, val_cost, lr)))
+                if select_by == 'sbd' and scores is not None and best_sbd.keep(scores[0]):
+                    torch.save(self.model.state_dict(), os.path.join(model_save_path, 'model_{}_sbd{}_{}.pth'.format(epoch, scores[0], lr)))
                 training_log_file.write('{},{}\n'.format(epoch, train_cost))
                 validation_log_file.write('{},{}\n'.format(epoch, val_cost))
                 training_log_file.flush()
@@ -333,6 +363,8 @@ class Model(object):
         if rank0:
             training_log_file.close()
             validation_log_file.close()
+            if scorer is not None:
+                scores_log_file.close()
         return history
 
     def __run_epoch(self, loader, clip_grad_norm, mode):
